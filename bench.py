@@ -20,6 +20,9 @@ LlamaBench.java:188-193) over a seeded synthetic GGUF-layout model of the real L
                (BASELINE.md section 3); a mismatch exits non-zero
 `--impl reference` times only that CPU restatement (the reference itself needs a JDK + TornadoVM,
 neither is installable here; see DESIGN.md).
+`--dump-outputs DIR` writes what the timed device loop computed (ids.npy: the greedy id of every timed step;
+logits.npy: the logits of the last timed step, single GPU only) so that two builds can be compared output
+for output: the model and the token stream are seeded, so the same arguments give the same inputs.
 """
 from __future__ import annotations
 
@@ -194,6 +197,15 @@ def parity_gate(plan, tokens, ref, want_logits: bool):
     return out
 
 
+def dump_outputs(d: str, ids, logits):
+    """What the timed device loop hands its caller (the greedy ids) plus the last step's logits (tensor-parallel ranks
+    hold only their slice of the vocabulary, so those are written only on one GPU)."""
+    os.makedirs(d, exist_ok=True)
+    np.save(os.path.join(d, "ids.npy"), np.asarray(ids, dtype=np.float64))
+    if logits is not None:
+        np.save(os.path.join(d, "logits.npy"), np.asarray(logits, dtype=np.float32))
+
+
 def main():
     global WORKLOAD, QUANT
     ap = argparse.ArgumentParser()
@@ -210,7 +222,14 @@ def main():
     ap.add_argument("--depth", type=int, default=-1, help="LlamaBench -d: KV positions filled before the timed steps (default: the warm-up steps)")
     ap.add_argument("--workload", default=WORKLOAD, choices=["llama-3-8b", "llama-3-70b", "llama-3.2-1b", "qwen3-4b"],
                     help="shape of the synthetic model (default: the BASELINE headline, Llama-3-8B; 70B is BASELINE config 5, meant for --gpus 2/4/8)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps write DIR/ids.npy (float64, greedy id of every timed step) and, on one GPU, "
+                         "DIR/logits.npy (float32, logits of the last timed step)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the timed GPU path; --impl reference times a bounded CPU sample")
     K, W = args.steps, max(args.warmup, 3)
     WORKLOAD = args.workload
     QUANT = args.quant
@@ -276,6 +295,8 @@ def main():
     barrier()
     ids, ms = plan.decode_sequence(tokens[D:D + K], K, D)
     barrier()
+    if args.dump_outputs and rank == 0:  # read back before the e2e leg and the kernel timings overwrite the logits buffer
+        dump_outputs(args.dump_outputs, ids, plan.read_buffer("logits", shape.vocab) if world == 1 else None)
     ms_rank = [ms]
     if world > 1:
         t = torch.tensor([ms], device=f"cuda:{local}")
