@@ -14,9 +14,6 @@ SOURCES = ["plan.cu"]
 
 def _deps():
     d = [os.path.join(CSRC, f) for f in os.listdir(CSRC) if f.endswith((".cu", ".cuh", ".h"))]
-    exp = os.path.join(CSRC, "experimental")
-    if os.path.isdir(exp):
-        d += [os.path.join(exp, f) for f in os.listdir(exp) if f.endswith((".cuh", ".h"))]
     d.append(os.path.join(HERE, "..", "include", "b200llama.h"))
     return d
 
@@ -29,21 +26,10 @@ NVCC_FLAGS = [
 ]
 
 
-STAMP = os.path.join(CSRC, ".build_defines")
-
-
-def _defines() -> list[str]:
-    """Opt-in experimental code paths: B200_NVCC_DEFINES="B200_SEQSUM_V2[,...]" (default: none)."""
-    return [d for d in os.environ.get("B200_NVCC_DEFINES", "").replace(",", " ").split() if d]
-
-
 def needs_build() -> bool:
     if not os.path.exists(LIB):
         return True
     t = os.path.getmtime(LIB)
-    built_with = open(STAMP).read().split() if os.path.exists(STAMP) else []
-    if built_with != _defines():
-        return True
     return any(os.path.getmtime(d) > t for d in _deps()) or os.path.getmtime(__file__) > t
 
 
@@ -51,7 +37,7 @@ def build(force: bool = False, verbose: bool = False) -> str:
     if not force and not needs_build():
         return LIB
     nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-    cmd = [nvcc, *NVCC_FLAGS, *[f"-D{d}" for d in _defines()], "-o", LIB, *[os.path.join(CSRC, s) for s in SOURCES], "-lcudart"]
+    cmd = [nvcc, *NVCC_FLAGS, "-o", LIB, *[os.path.join(CSRC, s) for s in SOURCES], "-lcudart"]
     r = subprocess.run(cmd, capture_output=True, text=True)
     if verbose or r.returncode != 0:
         sys.stderr.write(r.stdout + r.stderr)
@@ -59,8 +45,6 @@ def build(force: bool = False, verbose: bool = False) -> str:
         raise RuntimeError("nvcc failed building libb200llama.so")
     with open(os.path.join(CSRC, "ptxas.log"), "w") as f:
         f.write(r.stderr)
-    with open(STAMP, "w") as f:
-        f.write(" ".join(_defines()))
     return LIB
 
 

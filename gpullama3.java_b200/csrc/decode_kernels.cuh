@@ -13,7 +13,6 @@
 // but the arithmetic they implement is the CPU path's (InferenceCore.java:50-172, 565-697).
 #pragma once
 #include "common.cuh"
-#include "seqsum.cuh"
 #include "seqsum2.cuh"
 
 enum { MODE_STORE = 0, MODE_RESID = 1 };
@@ -39,32 +38,26 @@ __device__ __forceinline__ float emb_get(const DevMat &e, int token, int i) {
 // The sum is order-sensitive, so one thread walks it (squares precomputed in parallel).
 // One CTA.  Outputs: xq/xs (Q8_0 activation for the following matvec) and/or xb (float).
 // ------------------------------------------------------------------------------------------
-#define NORM_THREADS SEQSUM_THREADS
-static_assert(SEQSUM_THREADS == SEQSUM2_THREADS, "both accumulators run on the whole norm CTA");
+#define NORM_THREADS SEQSUM2_THREADS
 __host__ __device__ inline int norm_padded(int dim) { return (dim + SEQSUM2_THREADS - 1) / SEQSUM2_THREADS * SEQSUM2_THREADS; }
-// V2 = seqsum2.cuh (three scans + a short serial walk), otherwise the round-1 accumulator seqsum.cuh
-__host__ __device__ inline size_t norm_smem_bytes(int dim, bool v2) {
-    return v2 ? (size_t)norm_padded(dim) * 4 + 16 + seqsum2_scratch_bytes() : (size_t)dim * 4 + 16 + seqsum_scratch_bytes(dim);
-}
+// squares (padded to whole thread chunks) | the accumulator's scratch (seqsum2.cuh)
+__host__ __device__ inline size_t norm_smem_bytes(int dim) { return (size_t)norm_padded(dim) * 4 + 16 + seqsum2_scratch_bytes(); }
 
-template <bool EMBED, bool V2>
+template <bool EMBED>
 __global__ void __launch_bounds__(NORM_THREADS, 1) k_rmsnorm_quant(float *__restrict__ x, const StepState *__restrict__ st,
                                                                DevMat emb, const float *__restrict__ w, float eps, int dim,
                                                                int8_t *__restrict__ xq, float *__restrict__ xs,
-                                                               float *__restrict__ xb, long long *__restrict__ prof, TraceBuf tr, TpCtx tp, int tp_wait_op) {
+                                                               float *__restrict__ xb, TraceBuf tr, TpCtx tp, int tp_wait_op) {
     // One CTA of 1024 threads.  Under PDL this CTA only has to fit next to ONE streaming-matvec CTA
     // (the following matvec's CTA for this SM simply starts a little later).
     extern __shared__ __align__(16) float sm[];
     float *sq = sm;
     __shared__ float s_ss;
     const int tid = threadIdx.x;
-    long long t0 = 0, t1 = 0, t2 = 0, t3 = 0;
-    if (prof) t0 = clock64();
     trace_entry(tr);
     pdl_launch_dependents();
     pdl_wait();
     trace_mark(tr, 2);
-    if (prof) t1 = clock64();
     if (tp.n > 1 && tp_wait_op >= 0) { // x is gathered from all ranks: wait for their slices
         if (tid == 0) tp_wait(tp, TP_SLOT_X, tp_seq(tp, (unsigned)tp_wait_op));
         __syncthreads();
@@ -77,23 +70,11 @@ __global__ void __launch_bounds__(NORM_THREADS, 1) k_rmsnorm_quant(float *__rest
         else v = ldcg_f32c(x + i);
         sq[i] = __fmul_rn(v, v);
     }
-    if (V2)
-        for (int i = dim + tid; i < norm_padded(dim); i += NORM_THREADS) sq[i] = 0.0f;
+    for (int i = dim + tid; i < norm_padded(dim); i += NORM_THREADS) sq[i] = 0.0f;
     __syncthreads();
-    if (prof) t2 = clock64();
     // ss = sequential float sum of the squares (exact, parallel)
-    float ss;
-    int info0 = 0, info1 = 0, info2 = 0;
-    if (V2) {
-        SeqSum2Scratch scratch = seqsum2_carve(reinterpret_cast<unsigned char *>(sm + norm_padded(dim)));
-        ss = block_seqsum_exact_v2(sq, dim, scratch);
-        if (prof && tid == 0) { info0 = scratch.info[0]; info1 = scratch.info[1]; }
-    } else {
-        SeqSumScratch scratch = seqsum_carve(reinterpret_cast<unsigned char *>(sm + dim), dim);
-        ss = block_seqsum_exact(sq, dim, scratch, prof ? prof + 8 : nullptr);
-        if (prof && tid == 0) { info0 = scratch.info[0]; info1 = scratch.info[1]; info2 = scratch.info[2]; }
-    }
-    if (prof) t3 = clock64();
+    SeqSum2Scratch scratch = seqsum2_carve(reinterpret_cast<unsigned char *>(sm + norm_padded(dim)));
+    float ss = block_seqsum_exact_v2(sq, dim, scratch);
     if (EMBED) __threadfence_block(); // x[] written above by other threads of this block
     if (tid == 0) {
         ss = __fdiv_rn(ss, (float)dim);
@@ -131,27 +112,10 @@ __global__ void __launch_bounds__(NORM_THREADS, 1) k_rmsnorm_quant(float *__rest
         }
     }
     trace_mark(tr, 3);
-    if (prof) {
-        __syncthreads();
-        if (tid == 0) { long long t4 = clock64(); prof[0] = t1 - t0; prof[1] = t2 - t1; prof[2] = t3 - t2; prof[3] = t4 - t3;
-                        prof[4] = info0; prof[5] = info1; prof[6] = info2; }
-    }
 }
 
-// Test hooks: the sequential-sum emulations on arbitrary non-negative terms (padded with zeros: adding +0 never
-// changes a sum of non-negative floats).
-__global__ void __launch_bounds__(NORM_THREADS, 1) k_test_seqsum(const float *__restrict__ terms, int n, float *__restrict__ out, int *__restrict__ info) {
-    extern __shared__ __align__(16) float sm[];
-    float *sq = sm;
-    const int np = (n + 31) & ~31;
-    SeqSumScratch scratch = seqsum_carve(reinterpret_cast<unsigned char *>(sm + np), np);
-    for (int i = threadIdx.x; i < np; i += blockDim.x) sq[i] = i < n ? terms[i] : 0.0f;
-    if (threadIdx.x == 0) { scratch.info[0] = -1; scratch.info[1] = -2; }
-    __syncthreads();
-    float s = block_seqsum_exact(sq, np, scratch);
-    if (threadIdx.x == 0) { out[0] = s; info[0] = scratch.info[0]; info[1] = scratch.info[1]; }
-}
-// seqsum2.cuh with T threads (1024: the norm kernel's form; 256: the persistent decode kernel's form)
+// Test hook: the sequential-sum emulation on arbitrary non-negative terms (padded with zeros: adding +0 never
+// changes a sum of non-negative floats), seqsum2.cuh with T threads (1024: the norm kernel's form; 256: the persistent decode kernel's form)
 template <int T>
 __global__ void __launch_bounds__(T, 1) k_test_seqsum2(const float *__restrict__ terms, int n, float *__restrict__ out, int *__restrict__ info) {
     extern __shared__ __align__(16) float sm[];

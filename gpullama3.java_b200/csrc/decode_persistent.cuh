@@ -7,8 +7,8 @@
 //     warp, resident for the whole token;
 //   * the producer thread walks the tile-major weight stream of EVERY matrix of the token in consumption order (QKV, Wo,
 //     gate/up, W2 per layer, then lm_head) through one shared-memory ring of 1-D bulk copies: weight addresses never
-//     depend on activations, so HBM keeps streaming across what used to be kernel boundaries; when the ring is full
-//     (consumers stalled at a dependency) it keeps HBM busy by prefetching the next tiles into L2 (`l2_ahead`);
+//     depend on activations, so HBM keeps streaming across what used to be kernel boundaries; the copies carry an L2
+//     evict_first policy, so 8 GB of single-use weights per token do not push the KV rows, x and the norm weights out of L2;
 //   * phases are separated by epoch counters instead of kernel boundaries, five per layer:
 //         QKV rows -> attention | attention heads -> Wo | x -> ffn norm | hidden activation -> W2 | x -> next layer.
 //     Counters are monotone and never reset: target = (tick * layers + layer + 1) * arrivers, where tick counts launches.
@@ -75,11 +75,6 @@ struct PdArgs {
     float *att_scratch;        // [n_heads][ctx] score rows in global memory, or NULL: rows live in shared memory
     unsigned long long *trace; // [gridDim.x][n_layers + 1][PD_STAMPS] %globaltimer stamps, or NULL
     int with_logits;
-    unsigned l2_ahead;         // tiles the producer may prefetch into L2 beyond the ring while the ring is full
-    unsigned evict_first;      // 1: the weight stream's bulk copies carry an L2 evict_first policy -- 8 GB of single-use weights per token
-                               // otherwise churn the 126 MB L2 and push out the KV rows, x, the norm weights and the prefetched tiles
-    unsigned max_fly;          // experiment knob (B200_PD_MAXFLY): bulk copies one CTA keeps in flight; 0 = no limit but the ring (default:
-                               // limiting it never helped the dependent phases and always slowed the stream, profiles/r2_run3_knob_sweep.log)
     // tensor parallelism (tp.n == 1: everything below unused)
     TpCtx tp;
     unsigned pd_flags_off;     // offset of the persistent kernel's epoch flags [PD_S_SLOTS][TP_MAX] in every rank's comm buffer
@@ -93,7 +88,7 @@ struct PdSmem {
 
 // max_seg = widest column segment of any matrix of the plan; att_floats = 3*head_size + ctx when the score row lives in
 // shared memory, 3*head_size otherwise.
-__host__ __device__ inline PdSmem pd_layout(int dim, int qd, int hidden, int head_size, int att_floats, int max_seg, size_t budget, int max_stages = PD_MAX_STAGES) {
+__host__ __device__ inline PdSmem pd_layout(int dim, int qd, int hidden, int head_size, int att_floats, int max_seg, size_t budget) {
     PdSmem L;
     const int unit = smv_unit_bytes(max_seg);
     L.stage_bytes = (4 * unit + 127) & ~127;
@@ -125,7 +120,6 @@ __host__ __device__ inline PdSmem pd_layout(int dim, int qd, int hidden, int hea
     long room = (long)budget - (long)o;
     int s = room > 0 ? (int)(room / L.stage_bytes) : 0;
     if (s > PD_MAX_STAGES) s = PD_MAX_STAGES;
-    if (max_stages > 0 && s > max_stages) s = max_stages;
     L.stages = s;
     L.total = o + (size_t)s * L.stage_bytes;
     return L;
@@ -258,55 +252,18 @@ struct PdWalk {
     }
 };
 
-__device__ __forceinline__ bool mbar_try_wait(unsigned bar, unsigned parity) {
-    unsigned ok;
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n"
-        "selp.u32 %0, 1, 0, p;\n"
-        "}\n"
-        : "=r"(ok)
-        : "r"(bar), "r"(parity)
-        : "memory");
-    return ok != 0u;
-}
-
 __device__ __forceinline__ void pd_produce(const PdArgs &a, unsigned char *smem, const PdSmem &L, unsigned bar0) {
     const int S = L.stages;
     const unsigned long long pol = l2_policy_evict_first();
-    PdWalk cur, pf;
+    PdWalk cur;
     cur.init(&a);
-    pf = cur;
-    unsigned seq = 0, pf_seq = 0; // tiles issued into the ring / tiles covered by the L2 prefetch cursor
-    unsigned landed = 0;          // tiles known to have landed (their full barrier completed)
-    for (; cur.valid(); cur.next(), seq++) {
+    for (unsigned seq = 0; cur.valid(); cur.next(), seq++) {
         const int st = seq % S;
         const unsigned ph = (seq / S) & 1u;
-        const unsigned empty = bar0 + 8 * (PD_MAX_STAGES + st);
-        if (a.l2_ahead) {
-            // The slot is still occupied: the consumers are behind (stalled at a dependency).  Keep HBM busy by pulling
-            // the tiles beyond the ring into L2, at most l2_ahead tiles ahead of the ring's own requests.
-            while (!mbar_try_wait(empty, ph ^ 1u)) {
-                if (pf_seq < seq + (unsigned)S) { // the ring itself covers [seq, seq + S)
-                    while (pf_seq < seq + (unsigned)S && pf.valid()) { pf.next(); pf_seq++; }
-                }
-                if (pf.valid() && pf_seq < seq + (unsigned)S + a.l2_ahead) {
-                    bulk_prefetch_l2(pf.addr(), pf.tile_bytes);
-                    pf.next();
-                    pf_seq++;
-                }
-            }
-        } else mbar_wait(empty, ph ^ 1u);
-        if (a.max_fly) // in-flight throttle: wait for the oldest outstanding copy (its stage cannot have been re-armed: max_fly <= S)
-            while (seq - landed >= a.max_fly) {
-                mbar_wait(bar0 + 8 * (landed % S), (landed / S) & 1u);
-                landed++;
-            }
+        mbar_wait(bar0 + 8 * (PD_MAX_STAGES + st), ph ^ 1u); // slot free (first pass returns at once)
         const unsigned full = bar0 + 8 * st;
         mbar_expect_tx(full, cur.tile_bytes);
-        if (a.evict_first) bulk_g2s_evict_first(smem_u32(smem + L.off_ring + (size_t)st * L.stage_bytes), cur.addr(), cur.tile_bytes, full, pol);
-        else bulk_g2s(smem_u32(smem + L.off_ring + (size_t)st * L.stage_bytes), cur.addr(), cur.tile_bytes, full);
+        bulk_g2s_evict_first(smem_u32(smem + L.off_ring + (size_t)st * L.stage_bytes), cur.addr(), cur.tile_bytes, full, pol);
     }
 }
 

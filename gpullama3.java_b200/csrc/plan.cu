@@ -38,7 +38,6 @@ struct LayerW {
 // threads) -> async H2D on a copy stream -> device staging (double buffered) -> repack kernel on the plan's stream.  The host
 // copy of chunk i+1, the DMA of chunk i and the repack of the previous matrix overlap; nothing synchronises per matrix.
 struct Uploader {
-    bool on = false;
     cudaStream_t copy = nullptr;
     unsigned char *pin[2] = {nullptr, nullptr};
     size_t pin_bytes = 0;
@@ -97,12 +96,6 @@ struct b200_plan {
     cudaGraphExec_t g_pdecode = nullptr, g_pprefill = nullptr, g_ptrace = nullptr; // one persistent kernel per token (decode_persistent.cuh)
     unsigned long long *trace_rec = nullptr;
     int decode_mode = B200_DECODE_GRAPH; // which of the two the forward entry points launch
-    bool norm_v2 = false;                // k_rmsnorm_quant's accumulator: seqsum2.cuh instead of seqsum.cuh
-    // knobs read once at creation (never inside a launch helper)
-    size_t smv_budget = 96 * 1024;
-    int smv_budget_cols = 0;
-    unsigned l2_window = 0, pd_l2_ahead = 0, pd_max_fly = 0, pd_evict_first = 1;
-    int pd_max_stages = 0; // 0 = as many as shared memory holds
     float *att_scratch = nullptr; // [heads][ctx] score rows when the context does not fit shared memory
     int *smp_indices = nullptr, *smp_out = nullptr; // device-side sampler scratch (sampler.cuh): candidate list, {id, info[4]}
 
@@ -186,8 +179,6 @@ void par_memcpy(void *dst, const void *src, size_t n, int threads) {
 
 int up_init(b200_plan *p, size_t dst_bytes) {
     Uploader &u = p->up;
-    const char *e = getenv("B200_UPLOAD_SYNC"); // =1: the round-1 path (one blocking copy + synchronize per matrix)
-    if (e && e[0] == '1') return B200_OK;
     const char *t = getenv("B200_UPLOAD_THREADS");
     u.threads = t ? atoi(t) : 4;
     u.pin_bytes = (size_t)64 << 20;
@@ -200,7 +191,6 @@ int up_init(b200_plan *p, size_t dst_bytes) {
         CK(cudaEventCreateWithFlags(&u.d_ready[i], cudaEventDisableTiming));
         CK(cudaEventCreateWithFlags(&u.d_free[i], cudaEventDisableTiming));
     }
-    u.on = true;
     return B200_OK;
 }
 
@@ -217,7 +207,6 @@ void up_destroy(b200_plan *p) {
     }
     if (u.copy) cudaStreamDestroy(u.copy);
     u.copy = nullptr;
-    u.on = false;
 }
 
 // host bytes -> device, through the pinned double buffer, on the copy stream (asynchronous with respect to the caller except
@@ -290,7 +279,7 @@ static inline int eff_type(int t) { return kq_is_kquant(t) ? B200_GGML_Q8_0 : t;
 
 // Upload rows [0, rows) of a [rows][cols] GGUF matrix into dst at row offset `row_off`.  K-quant sources are re-quantised to Q8_0 on
 // the device (kquant.cuh) between the copy and the repack.
-int upload_matrix(b200_plan *p, const b200_tensor *t, int rows, int cols, DevMat &dst, int row_off, void *stage, size_t stage_bytes, int src_row = 0,
+int upload_matrix(b200_plan *p, const b200_tensor *t, int rows, int cols, DevMat &dst, int row_off, int src_row = 0,
                   int src_full_rows = -1) { // rows [src_row, src_row + rows) of a source tensor with src_full_rows rows (Phi-3's fused wqkv / gate-up)
     if (!t) return fail(p, B200_ERR_BAD_ARG, "missing tensor");
     if (src_full_rows < 0) src_full_rows = rows;
@@ -311,51 +300,42 @@ int upload_matrix(b200_plan *p, const b200_tensor *t, int rows, int cols, DevMat
         int8_t *qs = (int8_t *)dst.qs + (size_t)row_off * cols;
         __half *sc = (__half *)dst.sc + (size_t)row_off * (cols / 32);
         // chunked through the staging buffer (multiple of 34 bytes; of 8 blocks = one super-block for K-quants)
-        if (p->up.on) stage_bytes = p->up.dst_bytes;
-        const size_t q8_area = p->kq_off ? p->kq_off : stage_bytes;
+        const size_t q8_area = p->kq_off ? p->kq_off : p->up.dst_bytes;
         size_t blk_per_chunk = (q8_area / 34) & ~(size_t)7;
         for (size_t b0 = 0; b0 < nblk; b0 += blk_per_chunk) {
             size_t nb = nblk - b0 < blk_per_chunk ? nblk - b0 : blk_per_chunk;
             const unsigned char *hsrc = kq ? tdata + b0 / 8 * kb : tdata + b0 * 34;
             const size_t hbytes = kq ? nb / 8 * kb : nb * 34;
             int rc;
-            if (p->up.on) {
-                unsigned char *stg = nullptr;
-                if ((rc = up_stage_begin(p, &stg))) return rc;
-                if ((rc = up_h2d(p, stg + (kq ? p->kq_off : 0), hsrc, hbytes))) return rc;
-                if ((rc = up_stage_ready(p))) return rc;
-                stage = stg;
-            } else CK(cudaMemcpyAsync((unsigned char *)stage + (kq ? p->kq_off : 0), hsrc, hbytes, cudaMemcpyHostToDevice, p->stream));
+            unsigned char *stage = nullptr;
+            if ((rc = up_stage_begin(p, &stage))) return rc;
+            if ((rc = up_h2d(p, stage + (kq ? p->kq_off : 0), hsrc, hbytes))) return rc;
+            if ((rc = up_stage_ready(p))) return rc;
             if (kq) CK(launch_requant_kquant(t->ggml_type, (const unsigned char *)stage + p->kq_off, (unsigned char *)stage, (long long)nb, p->stream));
             size_t words = nb * 17;
             k_repack_q8<<<(unsigned)((words + 255) / 256), 256, 0, p->stream>>>((const uint16_t *)stage, (uint16_t *)(qs + b0 * 32),
                                                                                   (uint16_t *)(sc + b0), words);
             CK(cudaGetLastError());
-            if (p->up.on) { if ((rc = up_stage_release(p))) return rc; }
-            else CK(cudaStreamSynchronize(p->stream)); // staging buffer is reused
+            if ((rc = up_stage_release(p))) return rc;
         }
     } else {
         size_t esz = dst.type == B200_GGML_F16 ? 2 : 4;
-        if (p->up.on) return up_h2d(p, (uint8_t *)dst.qs + (size_t)row_off * cols * esz, tdata, (size_t)rows * cols * esz); // ordered by the final synchronize
-        CK(cudaMemcpy((uint8_t *)dst.qs + (size_t)row_off * cols * esz, tdata, (size_t)rows * cols * esz, cudaMemcpyHostToDevice));
+        return up_h2d(p, (uint8_t *)dst.qs + (size_t)row_off * cols * esz, tdata, (size_t)rows * cols * esz); // ordered by the final synchronize
     }
     return B200_OK;
 }
 
 // Upload up to three stacked GGUF Q8_0 matrices (or the gate/up pair) into tile-major layout.
 int upload_tiles(b200_plan *p, const b200_tensor *t0, const b200_tensor *t1, const b200_tensor *t2, int r0, int r1, int r2, int cols,
-                 bool gateup, TileMat &out, void *stage, size_t stage_bytes, const int *row0 = nullptr, const int *full = nullptr) {
+                 bool gateup, TileMat &out, const int *row0 = nullptr, const int *full = nullptr) {
     const b200_tensor *ts[3] = {t0, t1, t2};
     int rs[3] = {r0, r1, r2};
     RepackSrc src;
     size_t off = 0;
     int rc;
-    if (p->up.on) {
-        unsigned char *stg = nullptr;
-        if ((rc = up_stage_begin(p, &stg))) return rc;
-        stage = stg;
-        stage_bytes = p->up.dst_bytes;
-    }
+    unsigned char *stage = nullptr;
+    if ((rc = up_stage_begin(p, &stage))) return rc;
+    const size_t stage_bytes = p->up.dst_bytes;
     const size_t q8_area = p->kq_off ? p->kq_off : stage_bytes;
     size_t roff = 0; // cursor inside the raw (K-quant) area
     struct Requant { int type; const unsigned char *raw; unsigned char *q8; long long nblk; } rq[3];
@@ -380,20 +360,18 @@ int upload_tiles(b200_plan *p, const b200_tensor *t0, const b200_tensor *t1, con
             const size_t raw_row = (size_t)cols / 256 * kq_block_bytes(t->ggml_type), raw_bytes = (size_t)rs[k] * raw_row;
             const unsigned char *hsrc = (const unsigned char *)t->data + (size_t)first * raw_row;
             if (p->kq_off + roff + raw_bytes > stage_bytes) return fail(p, B200_ERR_STATE, "staging buffer too small");
-            unsigned char *rdst = (unsigned char *)stage + p->kq_off + roff;
-            if (p->up.on) { if ((rc = up_h2d(p, rdst, hsrc, raw_bytes))) return rc; }
-            else CK(cudaMemcpyAsync(rdst, hsrc, raw_bytes, cudaMemcpyHostToDevice, p->stream));
-            rq[n_rq++] = Requant{t->ggml_type, rdst, (unsigned char *)stage + off, (long long)rs[k] * (cols / 32)};
+            unsigned char *rdst = stage + p->kq_off + roff;
+            if ((rc = up_h2d(p, rdst, hsrc, raw_bytes))) return rc;
+            rq[n_rq++] = Requant{t->ggml_type, rdst, stage + off, (long long)rs[k] * (cols / 32)};
             roff += (raw_bytes + 255) & ~(size_t)255;
         } else {
             const unsigned char *hsrc = (const unsigned char *)t->data + (size_t)first * row_bytes;
-            if (p->up.on) { if ((rc = up_h2d(p, (unsigned char *)stage + off, hsrc, nbytes))) return rc; }
-            else CK(cudaMemcpyAsync((unsigned char *)stage + off, hsrc, nbytes, cudaMemcpyHostToDevice, p->stream));
+            if ((rc = up_h2d(p, stage + off, hsrc, nbytes))) return rc;
         }
-        src.raw[k] = (const unsigned char *)stage + off;
+        src.raw[k] = stage + off;
         off += (nbytes + 255) & ~(size_t)255;
     }
-    if (p->up.on && (rc = up_stage_ready(p))) return rc;
+    if ((rc = up_stage_ready(p))) return rc;
     for (int i = 0; i < n_rq; i++) CK(launch_requant_kquant(rq[i].type, rq[i].raw, rq[i].q8, rq[i].nblk, p->stream));
     src.gateup = gateup ? 1 : 0;
     const int rows = gateup ? r0 + r1 : r0 + r1 + r2;
@@ -409,9 +387,7 @@ int upload_tiles(b200_plan *p, const b200_tensor *t0, const b200_tensor *t1, con
     out.base = d;
     k_repack_tiles<<<(unsigned)((size_t)rows * out.nseg), 128, 0, p->stream>>>(src, d, rows, cols, out.seg, out.nseg, out.unit_bytes);
     CK(cudaGetLastError());
-    if (p->up.on) return up_stage_release(p);
-    CK(cudaStreamSynchronize(p->stream));
-    return B200_OK;
+    return up_stage_release(p);
 }
 
 int alloc_matrix(b200_plan *p, DevMat &m, int rows, int cols, int type) {
@@ -515,40 +491,19 @@ int launch_k(b200_plan *p, bool pdl, void (*kern)(KA...), dim3 grid, dim3 block,
 }
 
 const size_t SMV_SMEM_BUDGET_MAX = 96 * 1024;
-// Debug/tuning knobs, read ONCE per plan (b200_plan_create), never inside a launch helper.
+// Read ONCE per plan (b200_plan_create), never inside a launch helper.
 void read_knobs(b200_plan *p) {
-    const char *e = getenv("B200_SMV_BUDGET_KB");   // force a shallow ring
-    const char *m = getenv("B200_SMV_BUDGET_COLS"); // ... only for matrices with this many columns
-    size_t b = e ? (size_t)atoi(e) * 1024 : SMV_SMEM_BUDGET_MAX;
-    p->smv_budget = b > SMV_SMEM_BUDGET_MAX ? SMV_SMEM_BUDGET_MAX : b;
-    p->smv_budget_cols = m ? atoi(m) : 0;
-    const char *w = getenv("B200_L2_WINDOW_KB"); // experimental: measured slower on B200 (profiles/), off by default
-    p->l2_window = (unsigned)((w ? atoi(w) : 0) * 1024);
-    const char *a = getenv("B200_PD_L2_AHEAD"); // persistent kernel: tiles of L2 look-ahead while the ring is full
-    p->pd_l2_ahead = a ? (unsigned)atoi(a) : 0u;
-    const char *f = getenv("B200_PD_MAXFLY"); // persistent kernel: bulk copies in flight per CTA (0 = unlimited)
-    p->pd_max_fly = f ? (unsigned)atoi(f) : 0u; // measured (profiles/r2_run3_knob_sweep.log): any limit below the ring depth only slows the stream
-    const char *ev = getenv("B200_PD_EVICT_FIRST"); // persistent kernel: L2 evict_first policy on the weight stream (default on)
-    p->pd_evict_first = ev ? (unsigned)atoi(ev) : 1u;
-    const char *g = getenv("B200_PD_STAGES"); // persistent kernel: cap on the ring depth
-    p->pd_max_stages = g ? atoi(g) : 0;
-    const char *v = getenv("B200_NORM_V2");
-    p->norm_v2 = !(v && v[0] == '0');
     const char *d = getenv("B200_DECODE");
     // default: the CUDA graph -- measured faster than the persistent kernel on the same box (profiles/r2_final_a.log: 313.6 vs 285.1 tok/s,
     // 8B Q8_0; under tensor parallelism by 10-21 %).  B200_DECODE=persistent or b200_set_decode_mode select the one-kernel-per-token path.
     p->decode_mode = (d && !strcmp(d, "persistent")) ? B200_DECODE_PERSISTENT : B200_DECODE_GRAPH;
-}
-size_t smv_budget(const b200_plan *p, int cols) {
-    if (p->smv_budget_cols && cols && p->smv_budget_cols != cols) return SMV_SMEM_BUDGET_MAX;
-    return p->smv_budget;
 }
 
 template <int MODE>
 int launch_stream(b200_plan *p, const TileMat &W, const int8_t *xq, const float *xs, float *out, int8_t *hq, float *hs, bool argmax = false,
                   TraceBuf tr = TraceBuf{nullptr, 0, 0}, int wait_slot = -1, unsigned wait_op = 0, int out_slot = -1, unsigned out_op = 0,
                   int row_base = 0) {
-    SmvSmem L = smv_layout(W.cols, W.seg, smv_budget(p, W.cols));
+    SmvSmem L = smv_layout(W.cols, W.seg, SMV_SMEM_BUDGET_MAX);
     SmvArgs a;
     a.W = W; a.xq = xq; a.xs = xs; a.out = out; a.hq = hq; a.hs = hs; a.blk_cnt = p->blk_cnt;
     a.part_val = argmax ? p->part_val : nullptr;
@@ -556,7 +511,6 @@ int launch_stream(b200_plan *p, const TileMat &W, const int8_t *xq, const float 
     a.tr = tr;
     a.tp = p->tp;
     a.wait_slot = wait_slot; a.wait_op = wait_op; a.out_slot = out_slot; a.out_op = out_op; a.row_base = row_base;
-    a.l2_window = p->l2_window;
     return launch_k(p, p->use_pdl, k_stream_matvec_q8<MODE>, dim3(p->n_sms), dim3(SMV_THREADS), L.total, a, L);
 }
 
@@ -583,7 +537,7 @@ int enqueue_forward(b200_plan *p, bool with_logits, int *launches, bool trace = 
     const bool tpar = p->tp.n > 1;
     int n = 0;
     auto TR = [&](int id) { return TraceBuf{trace ? p->trace_rec : nullptr, n, id}; };
-    const size_t norm_smem = norm_smem_bytes(c.dim, p->norm_v2);
+    const size_t norm_smem = norm_smem_bytes(c.dim);
     int8_t *xq = q8 ? p->xq : nullptr;
     float *xs = q8 ? p->xs : nullptr;
     float *xbf = q8 ? nullptr : p->xb;
@@ -591,10 +545,9 @@ int enqueue_forward(b200_plan *p, bool with_logits, int *launches, bool trace = 
     const int rank = p->tp.rank;
     auto norm = [&](bool embed, const float *w, int wait_op) {
         auto go = [&](auto kern) {
-            return launch_k(p, pdl, kern, dim3(1), dim3(NORM_THREADS), norm_smem, p->x, (const StepState *)p->st, p->emb, w, c.rms_norm_eps, c.dim, xq, xs, xbf, (long long *)nullptr, TR(1), p->tp, wait_op);
+            return launch_k(p, pdl, kern, dim3(1), dim3(NORM_THREADS), norm_smem, p->x, (const StepState *)p->st, p->emb, w, c.rms_norm_eps, c.dim, xq, xs, xbf, TR(1), p->tp, wait_op);
         };
-        if (p->norm_v2) return embed ? go(k_rmsnorm_quant<true, true>) : go(k_rmsnorm_quant<false, true>);
-        return embed ? go(k_rmsnorm_quant<true, false>) : go(k_rmsnorm_quant<false, false>);
+        return embed ? go(k_rmsnorm_quant<true>) : go(k_rmsnorm_quant<false>);
     };
     for (int l = 0; l < c.n_layers; l++) {
         LayerW &L = p->layers[l];
@@ -691,7 +644,7 @@ int pd_prepare(b200_plan *p) {
     int maxdyn = 0;
     CK(cudaDeviceGetAttribute(&maxdyn, cudaDevAttrMaxSharedMemoryPerBlockOptin, p->device));
     const int att_floats = 3 * c.head_size + (p->att_scratch ? 0 : (c.context_length + PD_CT - 1) / PD_CT * PD_CT); // score row padded to whole accumulator chunks
-    const PdSmem L = pd_layout(c.dim, p->qd, c.hidden_dim, c.head_size, att_floats, max_seg, (size_t)maxdyn, p->pd_max_stages);
+    const PdSmem L = pd_layout(c.dim, p->qd, c.hidden_dim, c.head_size, att_floats, max_seg, (size_t)maxdyn);
     if (L.stages < 4) { p->pd_why = "shape leaves fewer than 4 ring stages of shared memory"; return B200_OK; }
     int rc;
     if (!p->pd_layers) {
@@ -732,9 +685,6 @@ int enqueue_persistent(b200_plan *p, bool with_logits, int *launches, bool trace
     a.part_val = p->part_val; a.part_idx = p->part_idx; a.sync = p->pd_sync; a.host_err = p->d_err;
     a.att_scratch = p->att_scratch; a.trace = trace ? p->pd_trace : nullptr;
     a.with_logits = with_logits ? 1 : 0;
-    a.l2_ahead = p->pd_l2_ahead;
-    a.evict_first = p->pd_evict_first;
-    a.max_fly = p->pd_max_fly > (unsigned)p->pd_L.stages ? (unsigned)p->pd_L.stages : p->pd_max_fly;
     a.tp = p->tp; a.pd_flags_off = p->pd_flags_off;
     a.head_base = p->tp.rank * p->nh_l; a.dim_base = p->tp.rank * p->dim_l; a.hid_base = p->tp.rank * p->hid_l; a.voc_base = p->tp.rank * p->voc_l;
     cudaLaunchConfig_t cfg = {};
@@ -804,7 +754,7 @@ int set_smem_attrs(b200_plan *p) {
     int maxdyn = 0;
     CK(cudaDeviceGetAttribute(&maxdyn, cudaDevAttrMaxSharedMemoryPerBlockOptin, p->device));
     if (c.dim > 8192) return fail(p, B200_ERR_UNSUPPORTED, "dim > 8192 not supported by the RMSNorm kernel");
-    size_t need_norm = norm_smem_bytes(c.dim, p->norm_v2);
+    size_t need_norm = norm_smem_bytes(c.dim);
     size_t need_att = att_smem_bytes(c.head_size, c.context_length, p->att_scratch != nullptr);
     int maxcols = c.hidden_dim > c.dim ? c.hidden_dim : c.dim;
     if (p->qd > maxcols) maxcols = p->qd;
@@ -815,10 +765,8 @@ int set_smem_attrs(b200_plan *p) {
         return fail(p, B200_ERR_UNSUPPORTED, "shape needs more shared memory than the device offers (%d bytes)", maxdyn);
     static bool done = false; // process-wide, like the attribute itself (plans are created from one thread at a time per process)
     if (done) return B200_OK;
-    CK(set_max_dyn(k_rmsnorm_quant<true, false>, maxdyn));
-    CK(set_max_dyn(k_rmsnorm_quant<false, false>, maxdyn));
-    CK(set_max_dyn(k_rmsnorm_quant<true, true>, maxdyn));
-    CK(set_max_dyn(k_rmsnorm_quant<false, true>, maxdyn));
+    CK(set_max_dyn(k_rmsnorm_quant<true>, maxdyn));
+    CK(set_max_dyn(k_rmsnorm_quant<false>, maxdyn));
     CK(set_max_dyn(k_attention<32>, maxdyn));
     CK(set_max_dyn(k_attention<64>, maxdyn));
     CK(set_max_dyn(k_attention<128>, maxdyn));
@@ -903,7 +851,6 @@ int build(b200_plan *p, const b200_tensor *tensors, int n_tensors) {
         p->use_pdl = (p->use_stream || p->use_f16_stream) && !(e2 && e2[0] == '0');
         if (c.tp_size > 1 && !p->use_stream) return fail(p, B200_ERR_UNSUPPORTED, "tensor parallelism needs the Q8_0 streaming path");
     }
-    void *stage = nullptr;
     size_t stage_bytes = (size_t)34 * (8u << 20); // 8 Mi blocks = 272 MiB
     if (p->use_stream) {
         size_t m1 = (size_t)c.vocab_size * c.dim, m2 = (size_t)2 * c.hidden_dim * c.dim, m3 = (size_t)(p->qd + 2 * p->kvd) * c.dim;
@@ -918,19 +865,18 @@ int build(b200_plan *p, const b200_tensor *tensors, int n_tensors) {
         stage_bytes *= 2;
     }
     const auto t_up0 = std::chrono::steady_clock::now();
-    if ((rc = up_init(p, stage_bytes))) return rc; // pipelined upload (B200_UPLOAD_SYNC=1: the blocking round-1 path)
-    if (!p->up.on && (p->wtype == B200_GGML_Q8_0 || eff_type(emb->ggml_type) == B200_GGML_Q8_0)) CK(cudaMalloc(&stage, stage_bytes));
-    struct StageGuard { void *s; b200_plan *pl; ~StageGuard() { if (s) cudaFree(s); up_destroy(pl); } } guard{stage, p};
+    if ((rc = up_init(p, stage_bytes))) return rc;
+    struct UploadGuard { b200_plan *pl; ~UploadGuard() { up_destroy(pl); } } guard{p};
 
     // embedding table (+ tied classifier: AbstractModelLoader.java:186-195)
     if ((rc = alloc_matrix(p, p->emb, c.vocab_size, c.dim, eff_type(emb->ggml_type)))) return rc;
-    if ((rc = upload_matrix(p, emb, c.vocab_size, c.dim, p->emb, 0, stage, stage_bytes))) return rc;
+    if ((rc = upload_matrix(p, emb, c.vocab_size, c.dim, p->emb, 0))) return rc;
     const b200_tensor *outw = find(tensors, n_tensors, "output.weight");
     if (p->use_stream) {
         if (!outw && eff_type(emb->ggml_type) != p->wtype) return fail(p, B200_ERR_UNSUPPORTED, "tied output weight type differs from the matrix type");
         {
             const int r0[3] = {c.tp_rank * p->voc_l, 0, 0}, fu[3] = {c.vocab_size, 0, 0};
-            if ((rc = upload_tiles(p, outw ? outw : emb, nullptr, nullptr, p->voc_l, 0, 0, c.dim, false, p->tout, stage, stage_bytes, r0, fu))) return rc;
+            if ((rc = upload_tiles(p, outw ? outw : emb, nullptr, nullptr, p->voc_l, 0, 0, c.dim, false, p->tout, r0, fu))) return rc;
         }
         p->out = p->emb;
         if ((rc = dalloc(p, &p->part_val, (size_t)p->n_sms * 4))) return rc;
@@ -943,7 +889,7 @@ int build(b200_plan *p, const b200_tensor *tensors, int n_tensors) {
             if ((rc = dalloc(p, &p->part_idx, (size_t)p->n_sms * 4 * 4))) return rc;
         }
         if ((rc = alloc_matrix(p, p->out, c.vocab_size, c.dim, p->wtype))) return rc;
-        if ((rc = upload_matrix(p, outw, c.vocab_size, c.dim, p->out, 0, stage, stage_bytes))) return rc;
+        if ((rc = upload_matrix(p, outw, c.vocab_size, c.dim, p->out, 0))) return rc;
     } else {
         if (eff_type(emb->ggml_type) != p->wtype) return fail(p, B200_ERR_UNSUPPORTED, "tied output weight type differs from the matrix type");
         p->out = p->emb;
@@ -976,42 +922,34 @@ int build(b200_plan *p, const b200_tensor *tensors, int n_tensors) {
         if (p->use_stream) {
             const int rk = c.tp_rank;
             const int qr0[3] = {rk * p->qd_l, k_src + rk * p->kvd_l, v_src + rk * p->kvd_l}, qfu[3] = {q_full, k_full, k_full};
-            if ((rc = upload_tiles(p, tq, tk, tv, p->qd_l, p->kvd_l, p->kvd_l, c.dim, false, L.tqkv, stage, stage_bytes, qr0, qfu))) return rc;
+            if ((rc = upload_tiles(p, tq, tk, tv, p->qd_l, p->kvd_l, p->kvd_l, c.dim, false, L.tqkv, qr0, qfu))) return rc;
             const int dr0[3] = {rk * p->dim_l, 0, 0}, dfu[3] = {c.dim, 0, 0};
-            if ((rc = upload_tiles(p, T("attn_output.weight"), nullptr, nullptr, p->dim_l, 0, 0, p->qd, false, L.two, stage, stage_bytes, dr0, dfu))) return rc;
+            if ((rc = upload_tiles(p, T("attn_output.weight"), nullptr, nullptr, p->dim_l, 0, 0, p->qd, false, L.two, dr0, dfu))) return rc;
             const int gr0[3] = {rk * p->hid_l, u_src + rk * p->hid_l, 0}, gfu[3] = {g_full, g_full, 0};
-            if ((rc = upload_tiles(p, tg, tu, nullptr, p->hid_l, p->hid_l, 0, c.dim, true, L.tgu, stage, stage_bytes, gr0, gfu))) return rc;
-            if ((rc = upload_tiles(p, T("ffn_down.weight"), nullptr, nullptr, p->dim_l, 0, 0, c.hidden_dim, false, L.tw2, stage, stage_bytes, dr0, dfu))) return rc;
+            if ((rc = upload_tiles(p, tg, tu, nullptr, p->hid_l, p->hid_l, 0, c.dim, true, L.tgu, gr0, gfu))) return rc;
+            if ((rc = upload_tiles(p, T("ffn_down.weight"), nullptr, nullptr, p->dim_l, 0, 0, c.hidden_dim, false, L.tw2, dr0, dfu))) return rc;
             continue;
         }
         // fused [Wq; Wk; Wv] so one launch produces the packed q|k|v vector
         if ((rc = alloc_matrix(p, L.qkv, p->qd + 2 * p->kvd, c.dim, p->wtype))) return rc;
-        if ((rc = upload_matrix(p, tq, p->qd, c.dim, L.qkv, 0, stage, stage_bytes, 0, q_full))) return rc;
-        if ((rc = upload_matrix(p, tk, p->kvd, c.dim, L.qkv, p->qd, stage, stage_bytes, k_src, k_full))) return rc;
-        if ((rc = upload_matrix(p, tv, p->kvd, c.dim, L.qkv, p->qd + p->kvd, stage, stage_bytes, v_src, k_full))) return rc;
+        if ((rc = upload_matrix(p, tq, p->qd, c.dim, L.qkv, 0, 0, q_full))) return rc;
+        if ((rc = upload_matrix(p, tk, p->kvd, c.dim, L.qkv, p->qd, k_src, k_full))) return rc;
+        if ((rc = upload_matrix(p, tv, p->kvd, c.dim, L.qkv, p->qd + p->kvd, v_src, k_full))) return rc;
         if ((rc = alloc_matrix(p, L.wo, c.dim, p->qd, p->wtype))) return rc;
-        if ((rc = upload_matrix(p, T("attn_output.weight"), c.dim, p->qd, L.wo, 0, stage, stage_bytes))) return rc;
+        if ((rc = upload_matrix(p, T("attn_output.weight"), c.dim, p->qd, L.wo, 0))) return rc;
         if ((rc = alloc_matrix(p, L.w1, c.hidden_dim, c.dim, p->wtype))) return rc;
-        if ((rc = upload_matrix(p, tg, c.hidden_dim, c.dim, L.w1, 0, stage, stage_bytes, 0, g_full))) return rc;
+        if ((rc = upload_matrix(p, tg, c.hidden_dim, c.dim, L.w1, 0, 0, g_full))) return rc;
         if ((rc = alloc_matrix(p, L.w3, c.hidden_dim, c.dim, p->wtype))) return rc;
-        if ((rc = upload_matrix(p, tu, c.hidden_dim, c.dim, L.w3, 0, stage, stage_bytes, u_src, g_full))) return rc;
+        if ((rc = upload_matrix(p, tu, c.hidden_dim, c.dim, L.w3, 0, u_src, g_full))) return rc;
         if ((rc = alloc_matrix(p, L.w2, c.dim, c.hidden_dim, p->wtype))) return rc;
-        if ((rc = upload_matrix(p, T("ffn_down.weight"), c.dim, c.hidden_dim, L.w2, 0, stage, stage_bytes))) return rc;
+        if ((rc = upload_matrix(p, T("ffn_down.weight"), c.dim, c.hidden_dim, L.w2, 0))) return rc;
     }
 
-    if (p->up.on) { // drain the pipeline: every copy and every repack has finished before the first forward
-        CK(cudaStreamSynchronize(p->up.copy));
-        CK(cudaStreamSynchronize(p->stream));
-    }
+    // drain the pipeline: every copy and every repack has finished before the first forward
+    CK(cudaStreamSynchronize(p->up.copy));
+    CK(cudaStreamSynchronize(p->stream));
     p->up.total_s = std::chrono::duration<double>(std::chrono::steady_clock::now() - t_up0).count();
-    {
-        const double hs = p->up.host_copy_s, ts = p->up.total_s;
-        const int64_t hb = p->up.h2d_bytes;
-        const bool was_on = p->up.on;
-        up_destroy(p); // pinned buffers and device staging are not needed any more
-        p->up.host_copy_s = hs; p->up.total_s = ts; p->up.h2d_bytes = hb; p->up.on = false;
-        (void)was_on;
-    }
+    up_destroy(p); // pinned buffers and device staging are not needed any more (the timings survive)
     // RoPE table exactly as RoPE.precomputeFreqsCis (RoPE.java:6-37, ropeScaling=false):
     // freq = (float)(1.0 / Math.pow(theta, i / (double) headSize)); val = pos * freq (float);
     // cos/sin evaluated in double and narrowed.
@@ -1127,7 +1065,7 @@ int prefill_init(b200_plan *p) {
     if (kv_mul > 64 || (kv_mul & (kv_mul - 1))) { c.why = "tensor-core prefill needs a power-of-two GQA ratio <= 64"; return B200_OK; }
     if (g.dim % 128 || p->qd % 128 || nqkv % 128 || g.hidden_dim % 64) { c.why = "tensor-core prefill needs dim, q width and q+k+v width multiples of 128, hidden a multiple of 64"; return B200_OK; }
     if (!pg::encode_fn()) { c.why = "cuTensorMapEncodeTiled not available from the driver"; return B200_OK; }
-    c.bpad = (c.batch + 511) / 512 * 512; // whole units of the widest GEMM tiling (two 256-row CTA-pair tiles)
+    c.bpad = (c.batch + 511) / 512 * 512; // a whole number of 256-row CTA-pair tiles
     int rc;
     if ((rc = dalloc(p, &c.X, (size_t)c.bpad * g.dim * 4))) return rc;
     if ((rc = dalloc(p, &c.QKV, (size_t)c.bpad * nqkv * 4))) return rc;
@@ -1158,23 +1096,10 @@ int prefill_init(b200_plan *p) {
     {
         const char *e = getenv("B200_GEMM_2CTA");
         c.pair = !(e && e[0] == '0') && nqkv % 256 == 0 && g.dim % 256 == 0 && g.hidden_dim % 128 == 0;
-        const char *e2 = getenv("B200_GEMM_PERSIST"); // persistent CTA-pair kernel (double-buffered TMEM) for QKV and gate/up: validated on the
-        c.persist = !(e2 && e2[0] == '0');
-        const char *e3 = getenv("B200_GEMM_PERSIST_RESID"); // =1: Wo / W2 through the persistent kernel too (split-K folded into its work list); experimental
-        c.persist_resid = c.persist && e3 && e3[0] == '1';            // GPU in round 2 (tests/test_gpu_prefill.py, profiles/r2_run1_first_green.log); =0 selects the one-tile kernels
     }
     if (!ok) { c.why = "cuTensorMapEncodeTiled rejected a tensor map"; return B200_OK; }
-    if (g.head_size == 128) {
-        CK(cudaFuncSetAttribute(k_pf_attention<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pa_smem_bytes<128>()));
-        CK(cudaFuncSetAttribute(k_pf_attention_mma<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pm_smem_bytes<128>()));
-    } else {
-        CK(cudaFuncSetAttribute(k_pf_attention<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pa_smem_bytes<64>()));
-        CK(cudaFuncSetAttribute(k_pf_attention_mma<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pm_smem_bytes<64>()));
-    }
-    {
-        const char *e = getenv("B200_PF_ATT");
-        c.att_simt = e && !strcmp(e, "simt");
-    }
+    if (g.head_size == 128) CK(cudaFuncSetAttribute(k_pf_attention_mma<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pm_smem_bytes<128>()));
+    else CK(cudaFuncSetAttribute(k_pf_attention_mma<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pm_smem_bytes<64>()));
     c.ready = true;
     c.mode = 1;
     c.why = "";
@@ -1222,26 +1147,14 @@ int prefill_forward(b200_plan *p, int n, int start_pos, int *launches) {
     constexpr int ST = pg::GEMM_STAGES, DEEP = pg::GEMM_STAGES_DEEP;
     // a GEMM that fits one wave has one CTA per SM anyway: give it the deep ring; otherwise two CTAs share an SM
     auto one_wave = [&](int n_tiles) { return mt * n_tiles <= p->n_sms; };
-    // CTA-pair path: M in 256-row pair tiles; the x += A W^T GEMMs (N = dim only) split K so that the grid fills the SMs --
-    // every split reduce-adds its partial product through TMA
-    const int mt2 = (n + 255) / 256 * 2, mt4 = (n + 511) / 512 * 4;
-    // gate/up (the one multi-wave GEMM): two pair tiles of M per CTA pair, so every weight tile is fetched once per 512 rows and
-    // the per-CTA prologue/epilogue is paid half as often (measured 108 vs 114 us at B = 512; for the one-wave split-K GEMMs the
-    // wider tile only lowers the CTA count -- measured slower -- so they keep one pair tile per pair)
-    const bool wide = n > 256;
+    // CTA-pair path: M in 256-row pair tiles; QKV and gate/up on the persistent kernel, the x += A W^T GEMMs (N = dim only) split K
+    // so that the grid fills the SMs -- every split reduce-adds its partial product through TMA
+    const int mt2 = (n + 255) / 256 * 2;
     auto pair_splits = [&](int n_tiles, int K) {
         const int ctas = mt2 * n_tiles, nk = K / pg::BK;
         int sp = p->n_sms / ctas;
         if (sp > 4) sp = 4;
         while (sp > 1 && nk / sp < 8) sp--;
-        return sp < 1 ? 1 : sp;
-    };
-    // persistent residual GEMMs: enough (tile, k-range) items for ~2 waves of the 74 clusters, at least 8 k-blocks per item
-    auto persist_splits = [&](int n_tiles, int K) {
-        const int tiles = (mt2 / 2) * n_tiles, nk = K / pg::BK, clusters = p->n_sms / 2;
-        int sp = (2 * clusters + tiles - 1) / tiles;
-        if (sp > 8) sp = 8;
-        while (sp > 1 && (nk / sp < 8 || (sp - 1) * ((nk + sp - 1) / sp) >= nk)) sp--;
         return sp < 1 ? 1 : sp;
     };
     k_pf_embed<<<n, 256, 0, s>>>(c.tok, p->emb, c.X, g.dim); nl++;
@@ -1250,37 +1163,30 @@ int prefill_forward(b200_plan *p, int n, int start_pos, int *launches) {
         const PrefillLayerMaps &m = c.maps[l];
         float *kc = p->key_cache + (size_t)l * ctx_kv, *vc = p->value_cache + (size_t)l * ctx_kv;
         k_pf_rmsnorm_f16<<<n, 256, 0, s>>>(c.X, L.attn_norm, g.rms_norm_eps, g.dim, c.A16); nl++;
-        if (c.pair && c.persist) { // round-2 candidate, B200_GEMM_PERSIST=1
+        if (c.pair) {
             if (pg::gemm2_persist_launch<pg::GEMM_F32, 256, pg::GEMM2_PERSIST_STAGES_256>(c.mA, m.qkv, m.qkv, c.mQKV, c.QKV, nqkv, n, mt2, nqkv / 256, g.dim, p->n_sms, s)) return fail(p, B200_ERR_CUDA, "QKV GEMM launch failed");
-        } else if (c.pair) {
-            if (pg::gemm2_launch<pg::GEMM_F32, 256, pg::GEMM2_STAGES_256>(c.mA, m.qkv, m.qkv, c.mQKV, c.QKV, nqkv, n, mt2, nqkv / 256, g.dim, s)) return fail(p, B200_ERR_CUDA, "QKV GEMM launch failed");
         } else
         if (one_wave(nqkv / pg::BN) ? pg::gemm_launch<pg::GEMM_F32, DEEP>(c.mA, m.qkv, m.qkv, c.mQKV, c.QKV, nqkv, n, mt, nqkv / pg::BN, g.dim, s)
                                     : pg::gemm_launch<pg::GEMM_F32, ST>(c.mA, m.qkv, m.qkv, c.mQKV, c.QKV, nqkv, n, mt, nqkv / pg::BN, g.dim, s))
             return fail(p, B200_ERR_CUDA, "QKV GEMM launch failed");
         nl++;
-        const int qt = PA_ROWS / kv_mul;
+        const int qt = PM_ROWS / kv_mul;
         const dim3 ag((n + qt - 1) / qt, g.n_kv_heads);
-        if (start_pos > 0 && !c.att_simt) { // rows written by earlier chunks / decode steps
+        if (start_pos > 0) { // rows written by earlier chunks / decode steps
             const size_t n4 = (size_t)start_pos * p->kvd / 4;
             k_pf_kv_to_f16<<<(unsigned)((n4 + 255) / 256 < 1184 ? (n4 + 255) / 256 : 1184), 256, 0, s>>>(kc, vc, c.KH, c.VH, n4);
             nl++;
         }
         if (g.head_size == 128) {
             k_pf_rope_kv<128><<<n, 256, 0, s>>>(c.QKV, nqkv, kc, vc, c.KH, c.VH, p->kvd, g.n_heads, g.n_kv_heads, p->kflags, L.q_norm, L.k_norm, g.rms_norm_eps, p->rope_cr, p->rope_ci, start_pos);
-            if (c.att_simt) k_pf_attention<128><<<ag, PA_THREADS, pa_smem_bytes<128>(), s>>>(c.QKV, nqkv, kc, vc, p->kvd, kv_mul, n, start_pos, inv_sqrt_hs, c.ATT16, p->qd);
-            else k_pf_attention_mma<128><<<ag, PM_THREADS, pm_smem_bytes<128>(), s>>>(c.QKV, nqkv, c.KH, c.VH, p->kvd, kv_mul, n, start_pos, inv_sqrt_hs, c.ATT16, p->qd);
+            k_pf_attention_mma<128><<<ag, PM_THREADS, pm_smem_bytes<128>(), s>>>(c.QKV, nqkv, c.KH, c.VH, p->kvd, kv_mul, n, start_pos, inv_sqrt_hs, c.ATT16, p->qd);
         } else {
             k_pf_rope_kv<64><<<n, 256, 0, s>>>(c.QKV, nqkv, kc, vc, c.KH, c.VH, p->kvd, g.n_heads, g.n_kv_heads, p->kflags, L.q_norm, L.k_norm, g.rms_norm_eps, p->rope_cr, p->rope_ci, start_pos);
-            if (c.att_simt) k_pf_attention<64><<<ag, PA_THREADS, pa_smem_bytes<64>(), s>>>(c.QKV, nqkv, kc, vc, p->kvd, kv_mul, n, start_pos, inv_sqrt_hs, c.ATT16, p->qd);
-            else k_pf_attention_mma<64><<<ag, PM_THREADS, pm_smem_bytes<64>(), s>>>(c.QKV, nqkv, c.KH, c.VH, p->kvd, kv_mul, n, start_pos, inv_sqrt_hs, c.ATT16, p->qd);
+            k_pf_attention_mma<64><<<ag, PM_THREADS, pm_smem_bytes<64>(), s>>>(c.QKV, nqkv, c.KH, c.VH, p->kvd, kv_mul, n, start_pos, inv_sqrt_hs, c.ATT16, p->qd);
         }
         nl += 2;
-        if (c.pair && c.persist_resid) { // persistent CTA-pair kernel with the split-K ranges folded into its work list
-            if (pg::gemm2_persist_launch<pg::GEMM_RESID, 256, pg::GEMM2_PERSIST_STAGES_256>(c.mATT, m.wo, m.wo, c.mX, c.X, g.dim, n, mt2, g.dim / 256, p->qd, p->n_sms, s, persist_splits(g.dim / 256, p->qd)))
-                return fail(p, B200_ERR_CUDA, "Wo GEMM launch failed");
-        } else if (c.pair) {
-            if (pg::gemm2_launch<pg::GEMM_RESID, 256, pg::GEMM2_STAGES_256>(c.mATT, m.wo, m.wo, c.mX, c.X, g.dim, n, mt2, g.dim / 256, p->qd, s, pair_splits(g.dim / 256, p->qd)))
+        if (c.pair) {
+            if (pg::gemm2_launch<256, pg::GEMM2_STAGES_256>(c.mATT, m.wo, c.mX, n, mt2, g.dim / 256, p->qd, s, pair_splits(g.dim / 256, p->qd)))
                 return fail(p, B200_ERR_CUDA, "Wo GEMM launch failed");
         } else
         if (one_wave(g.dim / pg::BN) ? pg::gemm_launch<pg::GEMM_RESID, DEEP>(c.mATT, m.wo, m.wo, c.mX, c.X, g.dim, n, mt, g.dim / pg::BN, p->qd, s)
@@ -1288,22 +1194,15 @@ int prefill_forward(b200_plan *p, int n, int start_pos, int *launches) {
             return fail(p, B200_ERR_CUDA, "Wo GEMM launch failed");
         nl++;
         k_pf_rmsnorm_f16<<<n, 256, 0, s>>>(c.X, L.ffn_norm, g.rms_norm_eps, g.dim, c.A16); nl++;
-        if (c.pair && c.persist) { // round-2 candidate, B200_GEMM_PERSIST=1
+        if (c.pair) {
             if (pg::gemm2_persist_launch<pg::GEMM_GATEUP, 256, pg::GEMM2_PERSIST_STAGES_256>(c.mA, m.w1p, m.w3p, c.mX, c.H16, g.hidden_dim, n, mt2, g.hidden_dim / 128, g.dim, p->n_sms, s)) return fail(p, B200_ERR_CUDA, "gate/up GEMM launch failed");
-        } else if (c.pair) {
-            if (wide ? pg::gemm2_launch<pg::GEMM_GATEUP, 256, pg::GEMM2_STAGES_256_M2, 2>(c.mA, m.w1p, m.w3p, c.mX, c.H16, g.hidden_dim, n, mt4, g.hidden_dim / 128, g.dim, s)
-                     : pg::gemm2_launch<pg::GEMM_GATEUP, 256, pg::GEMM2_STAGES_256>(c.mA, m.w1p, m.w3p, c.mX, c.H16, g.hidden_dim, n, mt2, g.hidden_dim / 128, g.dim, s))
-                return fail(p, B200_ERR_CUDA, "gate/up GEMM launch failed");
         } else
         if (one_wave(g.hidden_dim / (pg::BN / 2)) ? pg::gemm_launch<pg::GEMM_GATEUP, DEEP>(c.mA, m.w1, m.w3, c.mX, c.H16, g.hidden_dim, n, mt, g.hidden_dim / (pg::BN / 2), g.dim, s)
                                                   : pg::gemm_launch<pg::GEMM_GATEUP, ST>(c.mA, m.w1, m.w3, c.mX, c.H16, g.hidden_dim, n, mt, g.hidden_dim / (pg::BN / 2), g.dim, s))
             return fail(p, B200_ERR_CUDA, "gate/up GEMM launch failed");
         nl++;
-        if (c.pair && c.persist_resid) {
-            if (pg::gemm2_persist_launch<pg::GEMM_RESID, 256, pg::GEMM2_PERSIST_STAGES_256>(c.mH, m.w2, m.w2, c.mX, c.X, g.dim, n, mt2, g.dim / 256, g.hidden_dim, p->n_sms, s, persist_splits(g.dim / 256, g.hidden_dim)))
-                return fail(p, B200_ERR_CUDA, "W2 GEMM launch failed");
-        } else if (c.pair) {
-            if (pg::gemm2_launch<pg::GEMM_RESID, 256, pg::GEMM2_STAGES_256>(c.mH, m.w2, m.w2, c.mX, c.X, g.dim, n, mt2, g.dim / 256, g.hidden_dim, s, pair_splits(g.dim / 256, g.hidden_dim)))
+        if (c.pair) {
+            if (pg::gemm2_launch<256, pg::GEMM2_STAGES_256>(c.mH, m.w2, c.mX, n, mt2, g.dim / 256, g.hidden_dim, s, pair_splits(g.dim / 256, g.hidden_dim)))
                 return fail(p, B200_ERR_CUDA, "W2 GEMM launch failed");
         } else
         if (one_wave(g.dim / pg::BN) ? pg::gemm_launch<pg::GEMM_RESID, DEEP>(c.mH, m.w2, m.w2, c.mX, c.X, g.dim, n, mt, g.dim / pg::BN, g.hidden_dim, s)
@@ -1733,41 +1632,15 @@ int b200_trace_decode(b200_plan *p, int32_t token, int32_t position, uint64_t *r
     return B200_OK;
 }
 
-int b200_profile_norm(b200_plan *p, int64_t *cycles4) {
-    if (!p || !cycles4) return B200_ERR_BAD_ARG;
-    CK(cudaSetDevice(p->device));
-    long long *d = nullptr;
-    CK(cudaMalloc(&d, 128));
-    const b200_config &c = p->cfg;
-    const size_t norm_smem = norm_smem_bytes(c.dim, p->norm_v2);
-    const bool q8 = p->wtype == B200_GGML_Q8_0;
-    for (int i = 0; i < 3; i++)
-        if (p->norm_v2) k_rmsnorm_quant<false, true><<<1, NORM_THREADS, norm_smem, p->stream>>>(p->x, p->st, p->emb, p->layers[0].attn_norm, c.rms_norm_eps, c.dim,
-                                                                 q8 ? p->xq : nullptr, q8 ? p->xs : nullptr, q8 ? nullptr : p->xb, d, TraceBuf{nullptr, 0, 0}, p->tp, -1);
-        else k_rmsnorm_quant<false, false><<<1, NORM_THREADS, norm_smem, p->stream>>>(p->x, p->st, p->emb, p->layers[0].attn_norm, c.rms_norm_eps, c.dim,
-                                                                 q8 ? p->xq : nullptr, q8 ? p->xs : nullptr, q8 ? nullptr : p->xb, d, TraceBuf{nullptr, 0, 0}, p->tp, -1);
-    cudaError_t e = cudaStreamSynchronize(p->stream);
-    long long h[16] = {0};
-    if (e == cudaSuccess) e = cudaMemcpy(h, d, 128, cudaMemcpyDeviceToHost);
-    cudaFree(d);
-    for (int i = 0; i < 7; i++) cycles4[i] = h[i];
-    for (int i = 0; i < 5; i++) cycles4[8 + i] = h[9 + i] - h[8 + i]; // seqsum phases A, B, C, barrier, resolve
-    return e == cudaSuccess ? B200_OK : B200_ERR_CUDA;
-}
-
 static int run_seqsum_hook(const float *terms, int32_t n, int threads, float *out, int32_t *info) {
     if (!terms || !out || n <= 0 || n > 8192) return B200_ERR_BAD_ARG;
-    if (threads != 0 && threads != 256 && threads != 512 && threads != 1024) return B200_ERR_BAD_ARG;
+    if (threads != 256 && threads != 512 && threads != 1024) return B200_ERR_BAD_ARG;
     float *d = nullptr, *o = nullptr;
     if (cudaMalloc(&d, (size_t)n * 4) != cudaSuccess) return B200_ERR_OOM;
     if (cudaMalloc(&o, 16) != cudaSuccess) { cudaFree(d); return B200_ERR_OOM; }
     cudaError_t e = cudaMemcpy(d, terms, (size_t)n * 4, cudaMemcpyHostToDevice);
     if (e == cudaSuccess) {
-        if (threads == 0) { // round-1 accumulator (seqsum.cuh)
-            const size_t smem = (size_t)((n + 31) & ~31) * 4 + seqsum_scratch_bytes((n + 31) & ~31);
-            e = cudaFuncSetAttribute(k_test_seqsum, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-            if (e == cudaSuccess) k_test_seqsum<<<1, NORM_THREADS, smem>>>(d, n, o, reinterpret_cast<int *>(o) + 1);
-        } else if (threads == 1024) {
+        if (threads == 1024) {
             const size_t smem = (size_t)1024 * ((n + 1023) / 1024) * 4 + seqsum2_scratch_bytes(1024);
             e = cudaFuncSetAttribute(k_test_seqsum2<1024>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
             if (e == cudaSuccess) k_test_seqsum2<1024><<<1, 1024, smem>>>(d, n, o, reinterpret_cast<int *>(o) + 1);
@@ -1792,11 +1665,7 @@ static int run_seqsum_hook(const float *terms, int32_t n, int threads, float *ou
     return e == cudaSuccess ? B200_OK : B200_ERR_CUDA;
 }
 
-int b200_test_seqsum(const float *terms, int32_t n, float *out, int32_t *info) { return run_seqsum_hook(terms, n, 0, out, info); }
-int b200_test_seqsum2(const float *terms, int32_t n, int32_t threads, float *out, int32_t *info) {
-    if (threads != 256 && threads != 512 && threads != 1024) return B200_ERR_BAD_ARG;
-    return run_seqsum_hook(terms, n, threads, out, info);
-}
+int b200_test_seqsum2(const float *terms, int32_t n, int32_t threads, float *out, int32_t *info) { return run_seqsum_hook(terms, n, threads, out, info); }
 
 int b200_requant_kquant(int32_t ggml_type, const void *src, int64_t n_elems, void *dst_q8_0) {
     if (!src || !dst_q8_0 || n_elems <= 0 || n_elems % 256 || !kq_is_kquant(ggml_type)) return B200_ERR_BAD_ARG;
@@ -1813,9 +1682,11 @@ int b200_requant_kquant(int32_t ggml_type, const void *src, int64_t n_elems, voi
 
 int b200_gemm_f16(const uint16_t *a, const uint16_t *b, float *c, int32_t m, int32_t n, int32_t k, int32_t iters, float *ms) {
     const int stages = getenv("B200_GEMM_STAGES") ? atoi(getenv("B200_GEMM_STAGES")) : 0;
-    const int two_cta = getenv("B200_GEMM_2CTA") ? atoi(getenv("B200_GEMM_2CTA")) : 0; // 0, 128 or 256
+    const int two_cta = getenv("B200_GEMM_2CTA") ? atoi(getenv("B200_GEMM_2CTA")) : 0; // 0, 256 (with B200_GEMM_RESID) or 1256 (without)
     const int resid = getenv("B200_GEMM_RESID") ? atoi(getenv("B200_GEMM_RESID")) : 0; // C starts at 0 and accumulates over the timed launches
     if (!a || !b || !c || m <= 0 || n <= 0 || k <= 0 || m % 128 || n % 128 || k % 64) return B200_ERR_BAD_ARG;
+    // only the kernels the prefill launches (pg::gemm_f16)
+    if (two_cta ? two_cta != (resid ? 256 : 1256) : (stages != 0 && stages != 3 && stages != 6)) return B200_ERR_BAD_ARG;
     __half *da = nullptr, *db = nullptr;
     float *dc = nullptr;
     cudaEvent_t e0 = nullptr, e1 = nullptr;

@@ -7,7 +7,7 @@
 //   per layer:  A16 <- f16(rmsnorm(X) * w)                            k_pf_rmsnorm_f16   (batchedRmsReduce + batchedRmsApplyFP16)
 //               QKV <- A16 * [Wq;Wk;Wv]^T                             GEMM_F32           (gemmMMAQKV)
 //               q,k <- (Qwen3: per-head RMSNorm) RoPE; k,v -> cache   k_pf_rope_kv       (batchedRopeWithKVCachePacked)
-//               ATT16 <- causal softmax(q k^T / sqrt(hs)) v           k_pf_attention     (batchedFlashAttentionFP16Out)
+//               ATT16 <- causal softmax(q k^T / sqrt(hs)) v           k_pf_attention_mma (batchedFlashAttentionFP16Out)
 //               X += ATT16 * Wo^T                                     GEMM_RESID         (gemmMMA + residual)
 //               A16 <- f16(rmsnorm(X) * w)
 //               H16 <- f16(silu(A16 W1^T) * (A16 W3^T))               GEMM_GATEUP        (gemmMMAGateUp + batchedFFNSwiGLUFP16Packed)
@@ -34,9 +34,6 @@ struct PrefillCtx {
     bool ready = false; // tensor-core path usable for this plan
     int mode = 0;       // 0 = exact token-by-token graph, 1 = tensor-core GEMMs
     bool pair = true;      // CTA-pair (cta_group::2) GEMMs; B200_GEMM_2CTA=0 selects the single-CTA kernels
-    bool persist = true;   // persistent CTA-pair GEMM (double-buffered TMEM accumulators) for QKV and gate/up; B200_GEMM_PERSIST=0 turns it off
-    bool persist_resid = false; // B200_GEMM_PERSIST_RESID=1: the residual GEMMs (Wo, W2) through the persistent kernel with split-K work items
-    bool att_simt = false; // debug: FP32 SIMT attention instead of the mma.sync kernel (B200_PF_ATT=simt)
     float *X = nullptr, *QKV = nullptr;
     __half *A16 = nullptr, *ATT16 = nullptr, *H16 = nullptr;
     int *tok = nullptr;
@@ -157,140 +154,7 @@ __global__ void __launch_bounds__(256) k_pf_kv_to_f16(const float *__restrict__ 
     }
 }
 
-// ---- causal attention over the chunk + everything already in the cache ---------------------------
-// CTA = one KV head x a tile of QT = 64 / kv_mul query tokens -> 64 query rows (all query heads that share
-// the KV head), so each K/V tile read from L2 serves 64 rows.  FP32 SIMT flash attention: S = Q K^T into
-// shared memory, online softmax per row, O += P V in registers.  256 threads.
-constexpr int PA_THREADS = 256, PA_ROWS = 64, PA_KT = 64;
-template <int HS> constexpr size_t pa_smem_bytes() { return (size_t)(2 * PA_ROWS * (HS + 4) + PA_KT * HS + PA_ROWS * (PA_KT + 1) + 3 * PA_ROWS) * 4; }
-
-template <int HS>
-__global__ void __launch_bounds__(PA_THREADS) k_pf_attention(const float *__restrict__ qkv, int ldq, const float *__restrict__ kc, const float *__restrict__ vc,
-                                                            int kvd, int kv_mul, int n, int start_pos, float inv_sqrt_hs, __half *__restrict__ out, int ldo) {
-    extern __shared__ __align__(16) float pa_sm[];
-    constexpr int QP = HS + 4, SP = PA_KT + 1, CPT = HS / 32, H4 = HS / 4;
-    float *sQ = pa_sm, *sK = sQ + PA_ROWS * QP, *sV = sK + PA_ROWS * QP, *sS = sV + PA_KT * HS;
-    float *sM = sS + PA_ROWS * SP, *sL = sM + PA_ROWS, *sA = sL + PA_ROWS;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int QT = PA_ROWS / kv_mul, q0 = blockIdx.x * QT, g = blockIdx.y;
-
-    for (int idx = tid; idx < PA_ROWS * H4; idx += PA_THREADS) {
-        const int r = idx / H4, d4 = idx % H4, b = q0 + r / kv_mul, h = g * kv_mul + r % kv_mul;
-        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (b < n) {
-            v = *reinterpret_cast<const float4 *>(qkv + (size_t)b * ldq + h * HS + d4 * 4);
-            v.x *= inv_sqrt_hs; v.y *= inv_sqrt_hs; v.z *= inv_sqrt_hs; v.w *= inv_sqrt_hs;
-        }
-        *reinterpret_cast<float4 *>(sQ + r * QP + d4 * 4) = v;
-    }
-    if (tid < PA_ROWS) { sM[tid] = -INFINITY; sL[tid] = 0.0f; }
-    float acc[8][CPT];
-#pragma unroll
-    for (int rr = 0; rr < 8; rr++)
-#pragma unroll
-        for (int c = 0; c < CPT; c++) acc[rr][c] = 0.0f;
-
-    const int q_end = (q0 + QT < n ? q0 + QT : n);   // one past the last valid query token of the tile
-    const int nkeys = start_pos + q_end;             // keys 0 .. start_pos + q_end - 1 are visible to the last query
-    const int ty = tid >> 4, tx = tid & 15;
-#pragma unroll 1
-    for (int k0 = 0; k0 < nkeys; k0 += PA_KT) {
-        __syncthreads(); // previous tile fully consumed (also covers the Q / sM / sL initialisation)
-        for (int idx = tid; idx < PA_KT * H4; idx += PA_THREADS) {
-            const int j = idx / H4, d4 = idx % H4, t = k0 + j;
-            float4 kv = make_float4(0.f, 0.f, 0.f, 0.f), vv = kv;
-            if (t < nkeys) {
-                kv = *reinterpret_cast<const float4 *>(kc + (size_t)t * kvd + g * HS + d4 * 4);
-                vv = *reinterpret_cast<const float4 *>(vc + (size_t)t * kvd + g * HS + d4 * 4);
-            }
-            *reinterpret_cast<float4 *>(sK + j * QP + d4 * 4) = kv;
-            *reinterpret_cast<float4 *>(sV + j * HS + d4 * 4) = vv;
-        }
-        __syncthreads();
-        // S tile: thread (ty, tx) -> rows ty*4 .. +3, keys tx + 16 j
-        float s[4][4];
-#pragma unroll
-        for (int i = 0; i < 4; i++)
-#pragma unroll
-            for (int j = 0; j < 4; j++) s[i][j] = 0.0f;
-#pragma unroll 4
-        for (int d = 0; d < HS; d += 4) {
-            float4 qv[4], kv[4];
-#pragma unroll
-            for (int i = 0; i < 4; i++) qv[i] = *reinterpret_cast<const float4 *>(sQ + (ty * 4 + i) * QP + d);
-#pragma unroll
-            for (int j = 0; j < 4; j++) kv[j] = *reinterpret_cast<const float4 *>(sK + (tx + 16 * j) * QP + d);
-#pragma unroll
-            for (int i = 0; i < 4; i++)
-#pragma unroll
-                for (int j = 0; j < 4; j++) s[i][j] = fmaf(qv[i].w, kv[j].w, fmaf(qv[i].z, kv[j].z, fmaf(qv[i].y, kv[j].y, fmaf(qv[i].x, kv[j].x, s[i][j])))); // TU is built with -fmad=false
-        }
-#pragma unroll
-        for (int i = 0; i < 4; i++) {
-            const int r = ty * 4 + i, b = q0 + r / kv_mul;
-#pragma unroll
-            for (int j = 0; j < 4; j++) {
-                const int t = k0 + tx + 16 * j;
-                sS[r * SP + tx + 16 * j] = (b < n && t <= start_pos + b) ? s[i][j] : -INFINITY;
-            }
-        }
-        __syncthreads();
-        // online softmax: warp w owns rows w*8 .. w*8+7 (the same rows it accumulates below)
-#pragma unroll 1
-        for (int rr = 0; rr < 8; rr++) {
-            const int r = warp * 8 + rr;
-            const float v0 = sS[r * SP + lane], v1 = sS[r * SP + lane + 32];
-            float mx = fmaxf(v0, v1);
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-            const float m_old = sM[r], m_new = fmaxf(m_old, mx);
-            float p0 = 0.0f, p1 = 0.0f, alpha = 1.0f;
-            if (m_new != -INFINITY) {
-                p0 = expf(v0 - m_new);
-                p1 = expf(v1 - m_new);
-                alpha = expf(m_old - m_new);
-            }
-            float sum = p0 + p1;
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
-            sS[r * SP + lane] = p0;
-            sS[r * SP + lane + 32] = p1;
-            if (lane == 0) { sM[r] = m_new; sL[r] = sL[r] * alpha + sum; sA[r] = alpha; }
-        }
-        __syncthreads();
-#pragma unroll
-        for (int rr = 0; rr < 8; rr++) {
-            const float a = sA[warp * 8 + rr];
-#pragma unroll
-            for (int c = 0; c < CPT; c++) acc[rr][c] *= a;
-        }
-#pragma unroll 4
-        for (int j = 0; j < PA_KT; j++) {
-            float v[CPT];
-#pragma unroll
-            for (int c = 0; c < CPT; c++) v[c] = sV[j * HS + lane * CPT + c];
-#pragma unroll
-            for (int rr = 0; rr < 8; rr++) {
-                const float p = sS[(warp * 8 + rr) * SP + j];
-#pragma unroll
-                for (int c = 0; c < CPT; c++) acc[rr][c] = fmaf(p, v[c], acc[rr][c]);
-            }
-        }
-    }
-    __syncthreads();
-#pragma unroll
-    for (int rr = 0; rr < 8; rr++) {
-        const int r = warp * 8 + rr, b = q0 + r / kv_mul, h = g * kv_mul + r % kv_mul;
-        if (b < n) {
-            const float inv = 1.0f / sL[r];
-            __half *o = out + (size_t)b * ldo + h * HS + lane * CPT;
-#pragma unroll
-            for (int c = 0; c < CPT; c++) o[c] = __float2half_rn(acc[rr][c] * inv);
-        }
-    }
-}
-
-// ---- the same attention on the warp-level tensor cores ------------------------------------------
+// ---- causal attention over the chunk + everything already in the cache, on the warp-level tensor cores ----
 // FlashAttention-2 layout with mma.sync.m16n8k16 (f16 operands, f32 accumulation): CTA = one KV head x 64
 // query rows (4 warps x 16 rows), key tiles of 64.  Q (pre-scaled), K and V are converted to f16 on their
 // way into shared memory; S = Q K^T stays in registers, its accumulator layout is re-used directly as the

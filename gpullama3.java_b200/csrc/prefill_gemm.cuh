@@ -226,7 +226,7 @@ __global__ void __launch_bounds__(256) k_gemm_f16_tcgen05(const __grid_constant_
 // leader arms it (expect_tx for both CTAs' bytes), waits on it and issues the MMAs; tcgen05.commit with a
 // multicast mask frees the stage in both CTAs and finally publishes the accumulator (rows 0-127 in the
 // leader's TMEM, 128-255 in the peer's) to both epilogues, which are identical to the single-CTA ones.
-// GEMM_GATEUP: the leader's half of B is BN/2 rows of W1, the peer's half BN/2 rows of W3.
+// GEMM_GATEUP (persistent kernel below): the leader's half of B is BN/2 rows of W1, the peer's half BN/2 rows of W3.
 // =====================================================================================================
 __device__ __forceinline__ uint32_t cluster_ctarank() {
     uint32_t r;
@@ -257,22 +257,19 @@ __device__ __forceinline__ void umma_commit_2cta(uint32_t bar) { // arrives on t
     asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar), "h"(mask) : "memory");
 }
 
-// MT = 256-row pair tiles of M that one CTA pair computes against the SAME B tile (MT x BN TMEM columns): with MT = 2 a
-// 512-token chunk re-uses every weight tile for all its rows, so an SM ingests 32 + BN/4 KB per 2 x 128 x BN x 64 MACs
-// (170 FLOP/B at BN = 256 -- tensor-pipe bound instead of L2-ingest bound) and the fixed prologue/epilogue is paid once.
-template <int BN, int STAGES, int MT> constexpr size_t smem_bytes_2cta() {
-    return (size_t)STAGES * (MT * BM * BK * 2 + (BN / 2) * BK * 2) + (2 * STAGES + 1) * 8 + 16 + 1024;
+template <int BN, int STAGES> constexpr size_t smem_bytes_2cta() {
+    return (size_t)STAGES * (BM * BK * 2 + (BN / 2) * BK * 2) + (2 * STAGES + 1) * 8 + 16 + 1024;
 }
 
-template <int MODE, int BN, int STAGES, int MT>
+// x += A W^T for Wo and W2 (GEMM_RESID), split K over blockIdx.z: every split reduce-adds its partial product into x.
+template <int BN, int STAGES>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(256, 1)
-    k_gemm_f16_2cta(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_b, const __grid_constant__ CUtensorMap tma_b2,
-                    const __grid_constant__ CUtensorMap tma_c, void *__restrict__ Cv, int ldc, int m_valid, int K, int kb_per_split) {
+    k_gemm_f16_2cta(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_b, const __grid_constant__ CUtensorMap tma_c,
+                    int m_valid, int K, int kb_per_split) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t *smem = reinterpret_cast<uint8_t *>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-    constexpr int A1_BYTES = BM * BK * 2, A_BYTES = MT * A1_BYTES, B_BYTES = (BN / 2) * BK * 2; // per CTA and stage
-    constexpr int TCOLS = MT * BN;
-    static_assert(TCOLS == 128 || TCOLS == 256 || TCOLS == 512, "TMEM allocations are powers of two");
+    constexpr int A_BYTES = BM * BK * 2, B_BYTES = (BN / 2) * BK * 2; // per CTA and stage
+    static_assert(BN == 128 || BN == 256 || BN == 512, "TMEM allocations are powers of two");
     static_assert(STAGES * (A_BYTES + B_BYTES) >= BM * BN * 4, "the C tile is staged in the operand ring");
     uint8_t *sA = smem, *sB = smem + STAGES * A_BYTES;
     uint64_t *bars = reinterpret_cast<uint64_t *>(sB + STAGES * B_BYTES);
@@ -287,32 +284,29 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(256, 1)
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == 2) { // the same warp of both CTAs allocates the pair's accumulator columns
-        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s32(tmem_slot)), "r"((uint32_t)TCOLS) : "memory");
+        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s32(tmem_slot)), "r"((uint32_t)BN) : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     cluster_sync_all(); // barriers of both CTAs initialised before any remote complete_tx / commit can land
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const uint32_t tmem_base = *tmem_slot;
-    // split-K (GEMM_RESID only: every split reduce-adds its partial product into x): blockIdx.z owns k-blocks [kb0, kb0 + nk)
+    // split-K: blockIdx.z owns k-blocks [kb0, kb0 + nk)
     const int nk_all = (K + BK - 1) / BK, kb0 = blockIdx.z * kb_per_split;
     const int nk = nk_all - kb0 < kb_per_split ? nk_all - kb0 : kb_per_split;
-    // rows of this CTA in pair tile mt: m_base + mt * 256 + rank * 128 .. + 127
-    const int m_base = (int)(blockIdx.x >> 1) * (MT * 2 * BM) + (int)rank * BM;
-    const int n0 = blockIdx.y * (MODE == GEMM_GATEUP ? BN / 2 : BN);
+    // rows of this CTA: m0 .. m0 + 127 of the pair tile
+    const int m0 = (int)(blockIdx.x >> 1) * (2 * BM) + (int)rank * BM;
+    const int n0 = blockIdx.y * BN;
 
     if (warp == 0 && lane == 0) {
-        // ===== TMA producer (both CTAs): own A rows of every pair tile, own half of the B tile =====
-        const CUtensorMap *bmap = (MODE == GEMM_GATEUP && rank == 1) ? &tma_b2 : &tma_b;
-        const int brow = MODE == GEMM_GATEUP ? n0 : n0 + (int)rank * (BN / 2);
+        // ===== TMA producer (both CTAs): own A rows, own half of the B tile =====
+        const int brow = n0 + (int)rank * (BN / 2);
         for (int kb = 0; kb < nk; kb++) {
             const int st = kb % STAGES;
             mbar_wait(empty0 + 8 * st, ((kb / STAGES) & 1) ^ 1);
             if (rank == 0) mbar_expect_tx(full0 + 8 * st, 2 * (A_BYTES + B_BYTES));
-#pragma unroll
-            for (int mt = 0; mt < MT; mt++)
-                tma_load_2d_2sm(s32(sA + st * A_BYTES + mt * A1_BYTES), &tma_a, (kb0 + kb) * BK, m_base + mt * 2 * BM, full0 + 8 * st);
-            tma_load_2d_2sm(s32(sB + st * B_BYTES), bmap, (kb0 + kb) * BK, brow, full0 + 8 * st);
+            tma_load_2d_2sm(s32(sA + st * A_BYTES), &tma_a, (kb0 + kb) * BK, m0, full0 + 8 * st);
+            tma_load_2d_2sm(s32(sB + st * B_BYTES), &tma_b, (kb0 + kb) * BK, brow, full0 + 8 * st);
         }
     } else if (warp == 1 && lane == 0 && rank == 0) {
         // ===== MMA issuer: one thread of the leader CTA drives both SMs' tensor cores =====
@@ -321,99 +315,59 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(256, 1)
             const int st = kb % STAGES;
             mbar_wait(full0 + 8 * st, (kb / STAGES) & 1);
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            const uint64_t db = umma_desc_sw128(s32(sB + st * B_BYTES));
+            const uint64_t da = umma_desc_sw128(s32(sA + st * A_BYTES)), db = umma_desc_sw128(s32(sB + st * B_BYTES));
 #pragma unroll
-            for (int mt = 0; mt < MT; mt++) {
-                const uint64_t da = umma_desc_sw128(s32(sA + st * A_BYTES + mt * A1_BYTES));
-#pragma unroll
-                for (int k = 0; k < BK / 16; k++) umma_f16_2cta(tmem_base + (uint32_t)(mt * BN), da + 2 * k, db + 2 * k, idesc, (kb | k) != 0 ? 1u : 0u);
-            }
+            for (int k = 0; k < BK / 16; k++) umma_f16_2cta(tmem_base, da + 2 * k, db + 2 * k, idesc, (kb | k) != 0 ? 1u : 0u);
             umma_commit_2cta(empty0 + 8 * st);
         }
         umma_commit_2cta(tmem_full);
     }
     __syncwarp(); // the elected producer / MMA lanes rejoin their warps
     {
-        // ===== epilogue (both CTAs, own 128 rows of each pair tile): all 8 warps -- warp w reads TMEM lanes 32*(w%4).., warps 0-3
-        // take the first half of the columns and warps 4-7 the second =====
+        // ===== epilogue (both CTAs, own 128 rows): all 8 warps -- warp w reads TMEM lanes 32*(w%4).., warps 0-3 take the first
+        // half of the columns and warps 4-7 the second =====
         mbar_wait(tmem_full, 0);
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
         const int q = warp & 3, half = warp >> 2;
+        const int row = m0 + q * 32 + lane;
+        const uint32_t tlane = tmem_base + ((uint32_t)(q * 32) << 16);
+        if (m0 < m_valid) { // CTA-uniform: nothing of this tile is stored otherwise
+            const int rloc = q * 32 + lane;
 #pragma unroll 1
-        for (int mt = 0; mt < MT; mt++) {
-            const int m0 = m_base + mt * 2 * BM;
-            const int row = m0 + q * 32 + lane;
-            const uint32_t tlane = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(mt * BN);
-            if (MODE == GEMM_GATEUP) {
-                __half *C = reinterpret_cast<__half *>(Cv);
-#pragma unroll 1
-                for (int c0 = half * (BN / 4); c0 < (half + 1) * (BN / 4); c0 += 32) {
-                    uint32_t g[32], u[32];
-                    tmem_ld32(tlane + (uint32_t)c0, g);
-                    tmem_ld32(tlane + (uint32_t)(BN / 2 + c0), u);
-                    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-                    if (row < m_valid) {
-                        uint4 *dst = reinterpret_cast<uint4 *>(C + (size_t)row * ldc + n0 + c0);
+            for (int c = half * (BN / 64); c < (half + 1) * (BN / 64); c++) {
+                uint32_t r[32];
+                tmem_ld32(tlane + (uint32_t)(c * 32), r);
+                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+                uint8_t *buf = smem + c * (BM * 32 * 4) + rloc * 128;
 #pragma unroll
-                        for (int v = 0; v < 4; v++) {
-                            uint32_t w[4];
-#pragma unroll
-                            for (int e = 0; e < 4; e++) {
-                                const float g0 = __uint_as_float(g[8 * v + 2 * e]), g1 = __uint_as_float(g[8 * v + 2 * e + 1]);
-                                const float h0 = (g0 / (1.0f + expf(-g0))) * __uint_as_float(u[8 * v + 2 * e]);
-                                const float h1 = (g1 / (1.0f + expf(-g1))) * __uint_as_float(u[8 * v + 2 * e + 1]);
-                                const __half2 hh = __floats2half2_rn(h0, h1);
-                                w[e] = *reinterpret_cast<const uint32_t *>(&hh);
-                            }
-                            dst[v] = make_uint4(w[0], w[1], w[2], w[3]);
-                        }
-                    }
+                for (int j = 0; j < 8; j++) {
+                    uint4 o = make_uint4(r[4 * j], r[4 * j + 1], r[4 * j + 2], r[4 * j + 3]);
+                    if (row >= m_valid) o = make_uint4(0u, 0u, 0u, 0u);
+                    *reinterpret_cast<uint4 *>(buf + ((j ^ (rloc & 7)) << 4)) = o;
                 }
-            } else {
-                if (m0 >= m_valid) break; // CTA-uniform: nothing of this (and any later) pair tile is stored
-                const int rloc = q * 32 + lane;
-#pragma unroll 1
-                for (int c = half * (BN / 64); c < (half + 1) * (BN / 64); c++) {
-                    uint32_t r[32];
-                    tmem_ld32(tlane + (uint32_t)(c * 32), r);
-                    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-                    uint8_t *buf = smem + c * (BM * 32 * 4) + rloc * 128;
+            }
+            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+            __syncthreads();
+            if (threadIdx.x == 0) {
 #pragma unroll
-                    for (int j = 0; j < 8; j++) {
-                        uint4 o = make_uint4(r[4 * j], r[4 * j + 1], r[4 * j + 2], r[4 * j + 3]);
-                        if (row >= m_valid) o = make_uint4(0u, 0u, 0u, 0u);
-                        *reinterpret_cast<uint4 *>(buf + ((j ^ (rloc & 7)) << 4)) = o;
-                    }
+                for (int c = 0; c < BN / 32; c++) {
+                    const uint32_t src = s32(smem + c * (BM * 32 * 4));
+                    asm volatile("cp.reduce.async.bulk.tensor.2d.global.shared::cta.add.bulk_group [%0, {%2, %3}], [%1];" ::"l"(&tma_c), "r"(src),
+                                 "r"(n0 + c * 32), "r"(m0)
+                                 : "memory");
                 }
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                __syncthreads();
-                if (threadIdx.x == 0) {
-#pragma unroll
-                    for (int c = 0; c < BN / 32; c++) {
-                        const uint32_t src = s32(smem + c * (BM * 32 * 4));
-                        if (MODE == GEMM_RESID)
-                            asm volatile("cp.reduce.async.bulk.tensor.2d.global.shared::cta.add.bulk_group [%0, {%2, %3}], [%1];" ::"l"(&tma_c), "r"(src),
-                                         "r"(n0 + c * 32), "r"(m0)
-                                         : "memory");
-                        else
-                            asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(&tma_c), "r"(src),
-                                         "r"(n0 + c * 32), "r"(m0)
-                                         : "memory");
-                    }
-                    asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-                    asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); // also frees the staging buffer for the next pair tile
-                }
-                if (MT > 1) __syncthreads();
+                asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+                asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
             }
         }
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     cluster_sync_all(); // neither CTA may exit (or free TMEM) while the pair can still touch its shared memory / TMEM
-    if (warp == 2) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)TCOLS) : "memory");
+    if (warp == 2) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)BN) : "memory");
 }
 
 // =====================================================================================================
-// The CTA-pair GEMM as a PERSISTENT kernel (default for the QKV and gate/up GEMMs since round 2; B200_GEMM_PERSIST=0 disables).  One cluster per TPC walks tiles t = cluster + i * clusters (M pair tiles fastest, so neighbouring
+// The CTA-pair GEMM as a PERSISTENT kernel (the QKV and gate/up GEMMs).  One cluster per TPC walks tiles t = cluster + i * clusters (M pair tiles fastest, so neighbouring
 // clusters share a weight tile in L2); the accumulator is double buffered in TMEM (2 x BN columns), so while the four
 // epilogue warps drain tile i the MMA thread already accumulates tile i+1 and the producers are loading tile i+2 --
 // prologue, pipeline fill and epilogue no longer sit on the critical path of every tile (they are ~25 % of a K = 4096 tile
@@ -432,7 +386,7 @@ template <int BN, int STAGES> constexpr size_t smem_bytes_2cta_persist() {
 template <int MODE, int BN, int STAGES>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(256, 1)
     k_gemm_f16_2cta_persist(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_b, const __grid_constant__ CUtensorMap tma_b2,
-                            const __grid_constant__ CUtensorMap tma_c, void *__restrict__ Cv, int ldc, int m_valid, int K, int m_pairs, int n_tiles, int splits) {
+                            const __grid_constant__ CUtensorMap tma_c, void *__restrict__ Cv, int ldc, int m_valid, int K, int m_pairs, int n_tiles) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t *smem = reinterpret_cast<uint8_t *>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
     constexpr int A_BYTES = BM * BK * 2, B_BYTES = (BN / 2) * BK * 2, CST_BYTES = BM * 32 * 4;
@@ -457,28 +411,24 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(256, 1)
     cluster_sync_all();
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const uint32_t tmem_base = *tmem_slot;
-    // split-K (GEMM_RESID only: every split reduce-adds its partial product): a work item is (pair tile, k-range); items of one tile are
-    // adjacent in the walk so the B tile of neighbouring clusters differs only in k
-    const int nk_all = (K + BK - 1) / BK, nk_split = (nk_all + splits - 1) / splits;
-    const int n_clusters = (int)(gridDim.x >> 1), cid = (int)(blockIdx.x >> 1), total = m_pairs * n_tiles * splits;
+    const int nk = (K + BK - 1) / BK;
+    const int n_clusters = (int)(gridDim.x >> 1), cid = (int)(blockIdx.x >> 1), total = m_pairs * n_tiles;
 
     if (warp == 0 && lane == 0) {
         // ===== TMA producer (both CTAs) =====
         const CUtensorMap *bmap = (MODE == GEMM_GATEUP && rank == 1) ? &tma_b2 : &tma_b;
         int it = 0; // running k-block counter across tiles: the ring never drains between tiles
         for (int t = cid; t < total; t += n_clusters) {
-            const int ks = t % splits, tt = t / splits;
-            const int mp = tt % m_pairs, nt = tt / m_pairs;
+            const int mp = t % m_pairs, nt = t / m_pairs;
             const int m0 = mp * 2 * BM + (int)rank * BM;
             const int n0 = nt * (MODE == GEMM_GATEUP ? BN / 2 : BN);
             const int brow = MODE == GEMM_GATEUP ? n0 : n0 + (int)rank * (BN / 2);
-            const int kb0 = ks * nk_split, nk = min(nk_split, nk_all - kb0);
             for (int kb = 0; kb < nk; kb++, it++) {
                 const int st = it % STAGES;
                 mbar_wait(empty0 + 8 * st, ((it / STAGES) & 1) ^ 1);
                 if (rank == 0) mbar_expect_tx(full0 + 8 * st, 2 * (A_BYTES + B_BYTES));
-                tma_load_2d_2sm(s32(sA + st * A_BYTES), &tma_a, (kb0 + kb) * BK, m0, full0 + 8 * st);
-                tma_load_2d_2sm(s32(sB + st * B_BYTES), bmap, (kb0 + kb) * BK, brow, full0 + 8 * st);
+                tma_load_2d_2sm(s32(sA + st * A_BYTES), &tma_a, kb * BK, m0, full0 + 8 * st);
+                tma_load_2d_2sm(s32(sB + st * B_BYTES), bmap, kb * BK, brow, full0 + 8 * st);
             }
         }
     } else if (warp == 1 && lane == 0 && rank == 0) {
@@ -487,7 +437,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(256, 1)
         int it = 0, i = 0;
         for (int t = cid; t < total; t += n_clusters, i++) {
             const int buf = i & 1;
-            const int kb0 = (t % splits) * nk_split, nk = min(nk_split, nk_all - kb0);
             mbar_wait(tempty0 + 8 * buf, ((i >> 1) & 1) ^ 1); // both CTAs' epilogues have drained this buffer (first two uses pass at once)
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
             for (int kb = 0; kb < nk; kb++, it++) {
@@ -507,8 +456,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(256, 1)
         int i = 0, chunk = 0;                         // chunk: running count of staged 32-column chunks (staging buffer = chunk & 1)
         for (int t = cid; t < total; t += n_clusters, i++) {
             const int buf = i & 1;
-            const int tt = t / splits;
-            const int mp = tt % m_pairs, nt = tt / m_pairs;
+            const int mp = t % m_pairs, nt = t / m_pairs;
             const int m0 = mp * 2 * BM + (int)rank * BM;
             const int n0 = nt * (MODE == GEMM_GATEUP ? BN / 2 : BN);
             const int row = m0 + q * 32 + lane;
@@ -570,14 +518,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(256, 1)
                     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
                     asm volatile("bar.sync 2, 128;" ::: "memory");
                     if (et == 0) {
-                        if (MODE == GEMM_RESID)
-                            asm volatile("cp.reduce.async.bulk.tensor.2d.global.shared::cta.add.bulk_group [%0, {%2, %3}], [%1];" ::"l"(&tma_c), "r"(s32(cst)),
-                                         "r"(n0 + c * 32), "r"(m0)
-                                         : "memory");
-                        else
-                            asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(&tma_c), "r"(s32(cst)),
-                                         "r"(n0 + c * 32), "r"(m0)
-                                         : "memory");
+                        asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(&tma_c), "r"(s32(cst)),
+                                     "r"(n0 + c * 32), "r"(m0)
+                                     : "memory");
                         asm volatile("cp.async.bulk.commit_group;" ::: "memory");
                     }
                 }
@@ -644,29 +587,30 @@ inline int gemm_launch(const CUtensorMap &a, const CUtensorMap &b, const CUtenso
     return cudaGetLastError() == cudaSuccess ? 0 : -5;
 }
 
-// m_tiles = 128-row tiles of M, a multiple of 2 * MT (M padded to MT * 256).  B maps must have box rows = BN / 2.
-template <int MODE, int BN, int STAGES, int MT = 1>
-inline int gemm2_launch(const CUtensorMap &a, const CUtensorMap &b, const CUtensorMap &b2, const CUtensorMap &c, void *C, int ldc, int m_valid, int m_tiles,
-                        int n_tiles, int K, cudaStream_t stream, int splits = 1) {
+// x += A W^T through the CTA-pair kernel, K split `splits` ways.  m_tiles = 128-row tiles of M, even (M padded to 256).
+// B maps must have box rows = BN / 2.
+template <int BN, int STAGES>
+inline int gemm2_launch(const CUtensorMap &a, const CUtensorMap &b, const CUtensorMap &c, int m_valid, int m_tiles, int n_tiles, int K, cudaStream_t stream,
+                        int splits = 1) {
     static bool attr = false;
     if (!attr) {
-        if (cudaFuncSetAttribute(k_gemm_f16_2cta<MODE, BN, STAGES, MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes_2cta<BN, STAGES, MT>()) != cudaSuccess)
+        if (cudaFuncSetAttribute(k_gemm_f16_2cta<BN, STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes_2cta<BN, STAGES>()) != cudaSuccess)
             return -4;
         attr = true;
     }
-    if (m_tiles % (2 * MT) || splits < 1 || (splits > 1 && MODE != GEMM_RESID)) return -6;
+    if (m_tiles % 2 || splits < 1) return -6;
     const int nk = (K + BK - 1) / BK, per = (nk + splits - 1) / splits;
     if ((splits - 1) * per >= nk) return -6; // an empty split would publish an unwritten accumulator
-    k_gemm_f16_2cta<MODE, BN, STAGES, MT><<<dim3(m_tiles / MT, n_tiles, splits), 256, smem_bytes_2cta<BN, STAGES, MT>(), stream>>>(a, b, b2, c, C, ldc, m_valid, K, per);
+    k_gemm_f16_2cta<BN, STAGES><<<dim3(m_tiles, n_tiles, splits), 256, smem_bytes_2cta<BN, STAGES>(), stream>>>(a, b, c, m_valid, K, per);
     return cudaGetLastError() == cudaSuccess ? 0 : -5;
 }
-constexpr int GEMM2_STAGES_256 = 6, GEMM2_STAGES_128 = 8; // 192 KB of operand ring per CTA either way
-constexpr int GEMM2_STAGES_256_M2 = 4;                    // 4 x (32 KB of A + 16 KB of B)
+constexpr int GEMM2_STAGES_256 = 6; // 192 KB of operand ring per CTA
 
-// Persistent variant (round-2 candidate).  n_sms: SMs of the device; the grid is the largest even number of CTAs <= n_sms.
+// Persistent variant (GEMM_F32, GEMM_GATEUP).  n_sms: SMs of the device; the grid is the largest even number of CTAs <= n_sms.
 template <int MODE, int BN, int STAGES>
 inline int gemm2_persist_launch(const CUtensorMap &a, const CUtensorMap &b, const CUtensorMap &b2, const CUtensorMap &c, void *C, int ldc, int m_valid, int m_tiles,
-                                int n_tiles, int K, int n_sms, cudaStream_t stream, int splits = 1) {
+                                int n_tiles, int K, int n_sms, cudaStream_t stream) {
+    static_assert(MODE != GEMM_RESID, "the residual GEMMs run on k_gemm_f16_2cta");
     static bool attr = false;
     if (!attr) {
         if (cudaFuncSetAttribute(k_gemm_f16_2cta_persist<MODE, BN, STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes_2cta_persist<BN, STAGES>()) !=
@@ -674,16 +618,12 @@ inline int gemm2_persist_launch(const CUtensorMap &a, const CUtensorMap &b, cons
             return -4;
         attr = true;
     }
-    if (m_tiles & 1 || splits < 1 || (splits > 1 && MODE != GEMM_RESID)) return -6;
-    {
-        const int nk = (K + BK - 1) / BK, per = (nk + splits - 1) / splits;
-        if ((splits - 1) * per >= nk) return -6; // an empty split would publish an unwritten accumulator
-    }
-    const int m_pairs = m_tiles / 2, total = m_pairs * n_tiles * splits;
+    if (m_tiles & 1) return -6;
+    const int m_pairs = m_tiles / 2, total = m_pairs * n_tiles;
     int clusters = n_sms / 2;
     if (clusters > total) clusters = total;
     if (clusters < 1) return -6;
-    k_gemm_f16_2cta_persist<MODE, BN, STAGES><<<dim3(2 * clusters), 256, smem_bytes_2cta_persist<BN, STAGES>(), stream>>>(a, b, b2, c, C, ldc, m_valid, K, m_pairs, n_tiles, splits);
+    k_gemm_f16_2cta_persist<MODE, BN, STAGES><<<dim3(2 * clusters), 256, smem_bytes_2cta_persist<BN, STAGES>(), stream>>>(a, b, b2, c, C, ldc, m_valid, K, m_pairs, n_tiles);
     return cudaGetLastError() == cudaSuccess ? 0 : -5;
 }
 constexpr int GEMM2_PERSIST_STAGES_256 = 5; // 5 x 32 KB of operands + 2 x 16 KB of C staging
@@ -693,40 +633,28 @@ constexpr int GEMM2_PERSIST_STAGES_256 = 5; // 5 x 32 KB of operands + 2 x 16 KB
 constexpr int GEMM_STAGES = 3, GEMM_STAGES_DEEP = 6;
 
 // Test/measurement entry: C[M,N] (+)= A[M,K] * B[N,K]^T ; M, N multiples of 128, K multiple of 64.  Device pointers.
+// The kernels of the prefill: two_cta = 0: single-CTA F32 (resid = 0) or residual GEMM at `stages` = 3 or 6 (0 = 3);
+// two_cta = 256: the CTA-pair residual GEMM split `resid` ways over K; two_cta = 1256: the persistent CTA-pair F32 GEMM.
 inline int gemm_f16(const __half *A, const __half *B, float *C, int M, int N, int K, int stages, int resid, int two_cta, cudaStream_t stream) {
     if (M % BM || N % BN || K % BK) return -3;
     CUtensorMap ma, mb, mc;
     int rc;
-    if (two_cta) { // two_cta = pair-tile width (256 or 128)
-        const int bn = (two_cta == 512 || two_cta == 1256) ? 256 : two_cta;
-        if (M % 256 || N % bn) return -3;
+    if (two_cta) { // 256-wide pair tiles
+        if (M % 256 || N % 256) return -3;
         if ((rc = make_map(&ma, A, (uint64_t)M, (uint64_t)K, BM))) return rc;
-        if ((rc = make_map(&mb, B, (uint64_t)N, (uint64_t)K, bn / 2))) return rc;
+        if ((rc = make_map(&mb, B, (uint64_t)N, (uint64_t)K, 128))) return rc;
         if ((rc = make_map_c(&mc, C, (uint64_t)M, (uint64_t)N))) return rc;
-        if (two_cta == 1256) { // persistent CTA-pair kernel, 256-wide pair tiles (round-2 candidate)
-            int dev = 0, sms = 148;
-            cudaGetDevice(&dev);
-            cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-            return resid ? gemm2_persist_launch<GEMM_RESID, 256, GEMM2_PERSIST_STAGES_256>(ma, mb, mb, mc, C, N, M, M / BM, N / 256, K, sms, stream, resid)
-                         : gemm2_persist_launch<GEMM_F32, 256, GEMM2_PERSIST_STAGES_256>(ma, mb, mb, mc, C, N, M, M / BM, N / 256, K, sms, stream);
-        }
-        if (two_cta == 512) { // 256-wide pair tiles, two of them (512 rows) per CTA pair
-            if (M % 512) return -3;
-            return resid ? gemm2_launch<GEMM_RESID, 256, GEMM2_STAGES_256_M2, 2>(ma, mb, mb, mc, C, N, M, M / BM, N / 256, K, stream, resid)
-                         : gemm2_launch<GEMM_F32, 256, GEMM2_STAGES_256_M2, 2>(ma, mb, mb, mc, C, N, M, M / BM, N / 256, K, stream);
-        }
-        if (two_cta == 256)
-            return resid ? gemm2_launch<GEMM_RESID, 256, GEMM2_STAGES_256>(ma, mb, mb, mc, C, N, M, M / BM, N / 256, K, stream, resid)
-                         : gemm2_launch<GEMM_F32, 256, GEMM2_STAGES_256>(ma, mb, mb, mc, C, N, M, M / BM, N / 256, K, stream);
-        return resid ? gemm2_launch<GEMM_RESID, 128, GEMM2_STAGES_128>(ma, mb, mb, mc, C, N, M, M / BM, N / 128, K, stream)
-                     : gemm2_launch<GEMM_F32, 128, GEMM2_STAGES_128>(ma, mb, mb, mc, C, N, M, M / BM, N / 128, K, stream);
+        if (resid) return gemm2_launch<256, GEMM2_STAGES_256>(ma, mb, mc, M, M / BM, N / 256, K, stream, resid);
+        int dev = 0, sms = 148;
+        cudaGetDevice(&dev);
+        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+        return gemm2_persist_launch<GEMM_F32, 256, GEMM2_PERSIST_STAGES_256>(ma, mb, mb, mc, C, N, M, M / BM, N / 256, K, sms, stream);
     }
     if ((rc = make_map(&ma, A, (uint64_t)M, (uint64_t)K, BM))) return rc;
     if ((rc = make_map(&mb, B, (uint64_t)N, (uint64_t)K, BN))) return rc;
     if ((rc = make_map_c(&mc, C, (uint64_t)M, (uint64_t)N))) return rc;
     if (resid && stages == 6) return gemm_launch<GEMM_RESID, 6>(ma, mb, mb, mc, C, N, M, M / BM, N / BN, K, stream);
     if (resid) return gemm_launch<GEMM_RESID, GEMM_STAGES>(ma, mb, mb, mc, C, N, M, M / BM, N / BN, K, stream);
-    if (stages == 4) return gemm_launch<GEMM_F32, 4>(ma, mb, mb, mc, C, N, M, M / BM, N / BN, K, stream);
     if (stages == 6) return gemm_launch<GEMM_F32, 6>(ma, mb, mb, mc, C, N, M, M / BM, N / BN, K, stream);
     return gemm_launch<GEMM_F32, GEMM_STAGES>(ma, mb, mb, mc, C, N, M, M / BM, N / BN, K, stream);
 }

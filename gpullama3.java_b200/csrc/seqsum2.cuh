@@ -1,12 +1,15 @@
 // seqsum2.cuh -- the exact sequential-sum accumulator of the decode path's RMSNorms (round 2; the algorithm is validated on
 // the CPU by tools/seqsum2/proto.c, on the GPU by tools/seqsum2/harness.cu and tests/test_gpu_parity.py).
 //
-// Same contract as block_seqsum_exact (seqsum.cuh): the bit-exact value of  s = 0; for (i) s = s + t[i]  for non-negative
-// float terms (InferenceCore.rmsnorm's accumulator, InferenceCore.java:39-48), evaluated by one CTA.  Where the round-1
-// kernel works in 32-term groups with per-warp ordered composition, entry lists and a literal first quarter (~16 us at
-// n = 4096, a third of the decode step), this version is three block-wide scans and a ~25-item serial walk:
+// The bit-exact value of  s = 0; for (i) s = s + t[i]  for non-negative float terms (InferenceCore.rmsnorm's accumulator,
+// InferenceCore.java:39-48), evaluated by one CTA.  Float addition is not associative, so a tree reduction gives different
+// bits, and a literal chain costs ~8-10 cycles per term on one thread.  While the running sum s stays inside one binade
+// [2^e, 2^(e+1)) its mantissa M is an integer in units of u = 2^(e-23), and adding a term t rounds to  M + k + [f > 1/2]
+// with t/u = k + f (on an exact tie, f == 1/2, round-half-even makes the increment depend on the parity of M).  So inside a
+// binade a step is the integer map  M -> M + a[M & 1], and such maps compose associatively.  The sum is three block-wide
+// scans and a ~25-item serial walk:
 //   1. float prefix P over per-thread sums (E consecutive terms per thread)            -> predicted binade per thread
-//   2. a thread whose P range lies well inside one binade composes its E steps  M -> M + a[M & 1]  (seqsum.cuh: SeqPair)
+//   2. a thread whose P range lies well inside one binade composes its E steps  M -> M + a[M & 1]  (SeqPair)
 //      into one pair ("clean"); any other thread is "literal"
 //   3. segmented scan of the pairs over runs of clean threads with equal binade          (pairs compose associatively)
 //   4. item list (ballot/popc compaction): one item per literal thread and one per run
@@ -14,10 +17,47 @@
 //      exit) and add the integer; a failed check replays the run literally.  Predictions decide speed, never the result.
 // CPU model (20000 adversarial cases, n = 2048/4096/8192): 0 mismatches, ~3 head threads + ~24 items per sum.
 #pragma once
-#include "seqsum.cuh"
+#include "common.cuh"
 
 #define SEQSUM2_THREADS 1024
 #define SEQSUM2_LITERAL INT_MIN
+
+struct SeqPair { // the step  M -> M + a[M & 1]
+    unsigned a0, a1;
+};
+__device__ __forceinline__ SeqPair seq_compose(SeqPair L, SeqPair R) { // apply L, then R
+    SeqPair o;
+    o.a0 = L.a0 + ((L.a0 & 1u) ? R.a1 : R.a0);
+    o.a1 = L.a1 + (((1u + L.a1) & 1u) ? R.a1 : R.a0);
+    o.a0 = min(o.a0, 1u << 26); // saturate: anything >= 2^24 fails verification anyway
+    o.a1 = min(o.a1, 1u << 26);
+    return o;
+}
+
+__device__ __forceinline__ int f32_exponent(float f) { return (int)((__float_as_uint(f) >> 23) & 0xffu) - 127; }
+
+// Parity pair of adding t to a running sum in binade e (ulp 2^(e-23)).  Returns false when t >= 2^(e+1)
+// (not a within-binade step).
+__device__ __forceinline__ bool seq_pair(float t, int e, SeqPair &pr) {
+    const unsigned tb = __float_as_uint(t);
+    const int et = (int)(tb >> 23);
+    pr.a0 = pr.a1 = 0u;
+    if (et == 0) return true; // zero / denormal term: far below half an ulp (e >= -90)
+    const unsigned m = (tb & 0x7fffffu) | 0x800000u;
+    int shift = (e + 127) - et; // t / ulp = m * 2^-shift
+    if (shift < 0) return false;
+    if (shift > 25) shift = 25;
+    const unsigned k = m >> shift;
+    const unsigned rem = m & ((1u << shift) - 1u);
+    const unsigned half = shift ? (1u << (shift - 1)) : 0u;
+    if (shift && rem == half) { // exact tie: the result mantissa M + k + r must be even
+        pr.a0 = k + (k & 1u);
+        pr.a1 = k + ((k + 1u) & 1u);
+    } else {
+        pr.a0 = pr.a1 = k + ((shift && rem > half) ? 1u : 0u);
+    }
+    return true;
+}
 
 struct SeqItem {
     int cls;          // SEQSUM2_LITERAL or the binade of a run
@@ -263,7 +303,7 @@ __device__ float block_seqsum_exact_v2_t(const float *sq, int n, SeqSum2Scratch 
     return sc.result[0];
 }
 
-// The whole-CTA form used by k_rmsnorm_quant (B200_SEQSUM_V2): SEQSUM2_THREADS threads, __syncthreads.
+// The whole-CTA form used by k_rmsnorm_quant: SEQSUM2_THREADS threads, __syncthreads.
 __device__ __forceinline__ float block_seqsum_exact_v2(const float *sq, int n, SeqSum2Scratch sc) {
     return block_seqsum_exact_v2_t<SEQSUM2_THREADS>(sq, n, sc, (int)threadIdx.x, SeqSum2BlockSync());
 }

@@ -90,12 +90,7 @@ __device__ __forceinline__ void mbar_wait(unsigned bar, unsigned parity) {
         "}\n" ::"r"(bar), "r"(parity)
         : "memory");
 }
-__device__ __forceinline__ void bulk_g2s(unsigned dst, const void *src, unsigned bytes, unsigned bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst), "l"(src),
-                 "r"(bytes), "r"(bar)
-                 : "memory");
-}
-// The same copy with an L2 evict_first policy: single-use weight tiles must not push the KV rows, activations and norm weights out of L2
+// Global -> shared bulk copy with an L2 evict_first policy: single-use weight tiles must not push the KV rows, activations and norm weights out of L2
 // (measured on the persistent kernel: +6 % tokens/s, profiles/r2_run6_evict_first_qwen3.log).
 __device__ __forceinline__ unsigned long long l2_policy_evict_first() {
     unsigned long long pol;
@@ -106,11 +101,6 @@ __device__ __forceinline__ void bulk_g2s_evict_first(unsigned dst, const void *s
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;" ::"r"(dst), "l"(src),
                  "r"(bytes), "r"(bar), "l"(pol)
                  : "memory");
-}
-// Pull a span of (immutable) weights into L2 without occupying shared memory: lets a kernel that is
-// resident but still waiting for its dependency keep HBM busy far beyond its smem ring.
-__device__ __forceinline__ void bulk_prefetch_l2(const void *src, unsigned bytes) {
-    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src), "r"(bytes) : "memory");
 }
 __device__ __forceinline__ void consumer_bar_sync() { asm volatile("bar.sync 1, %0;" ::"n"(SMV_CONSUMER_WARPS * 32) : "memory"); }
 
@@ -165,7 +155,6 @@ struct SmvArgs {
     float *part_val;    // STORE (lm_head): per-CTA running maximum of the rows it produced ...
     int *part_idx;      // ... and the lowest row index attaining it (FloatTensor.argmax tie-break), or NULL
     TraceBuf tr;
-    unsigned l2_window; // bytes of this CTA's slice to keep prefetched into L2 ahead of the ring (0 = off)
     // tensor parallelism (tp.n == 1: unused)
     TpCtx tp;
     int wait_slot;      // slot whose flags gate the activation (-1: none)
@@ -209,25 +198,13 @@ __global__ void __launch_bounds__(SMV_THREADS, 1) k_stream_matvec_q8(SmvArgs a, 
         if (lane == 0) {
             unsigned seq = 0;
             const unsigned long long pol = l2_policy_evict_first();
-            // L2 prefetch cursor over this CTA's contiguous slice (memory order; the ring consumes the same
-            // bytes round by round), kept at most a.l2_window bytes ahead of what the ring has requested.
-            const unsigned char *slice = W.base + (size_t)g0 * nseg * tile_bytes;
-            const size_t slice_bytes = (size_t)(g1 - g0) * nseg * tile_bytes;
-            size_t pf = 0;
             for (int gb = g0; gb < g1; gb += SMV_CONSUMER_WARPS) {
                 int nw = min(SMV_CONSUMER_WARPS, g1 - gb);
                 for (int s = 0; s < nseg; s++)
+#pragma unroll 1 // one copy per iteration: the producer is a single thread, its code size is what matters
                     for (int w = 0; w < nw; w++, seq++) {
                         int st = seq % S;
                         unsigned ph = (seq / S) & 1u;
-                        if (a.l2_window) {
-                            const size_t issued = (size_t)seq * tile_bytes;
-                            if (pf < issued) pf = issued;
-                            while (pf < slice_bytes && pf < issued + a.l2_window) {
-                                bulk_prefetch_l2(slice + pf, tile_bytes);
-                                pf += tile_bytes;
-                            }
-                        }
                         mbar_wait(bar0 + 8 * (SMV_MAX_STAGES + st), ph ^ 1u); // slot free (first pass returns at once)
                         unsigned full = bar0 + 8 * st;
                         mbar_expect_tx(full, tile_bytes);

@@ -41,7 +41,7 @@ class Tensor(C.Structure):
 
 EXPORTS = ["b200_plan_create", "b200_forward_decode", "b200_forward_prefill", "b200_forward_batch_prefill", "b200_set_prefill_mode", "b200_prefill_info",
            "b200_set_decode_mode", "b200_decode_info", "b200_trace_persistent", "b200_test_seqsum2", "b200_forward_decode_sample", "b200_upload_info", "b200_requant_kquant",
-           "b200_decode_sequence", "b200_time_kernel", "b200_tp_handle", "b200_tp_attach", "b200_trace_decode", "b200_profile_norm", "b200_test_seqsum", "b200_gemm_f16", "b200_kv_reset", "b200_read_buffer", "b200_launches_per_decode",
+           "b200_decode_sequence", "b200_time_kernel", "b200_tp_handle", "b200_tp_attach", "b200_trace_decode", "b200_gemm_f16", "b200_kv_reset", "b200_read_buffer", "b200_launches_per_decode",
            "b200_device_bytes", "b200_plan_free", "b200_last_error", "b200_version"]
 
 _lib = None
@@ -63,11 +63,9 @@ def lib() -> C.CDLL:
     L.b200_forward_batch_prefill.argtypes = [vp, vp, i32, i32]
     L.b200_decode_sequence.argtypes = [vp, vp, i32, i32, i32, vp, C.POINTER(C.c_float)]
     L.b200_kv_reset.argtypes = [vp]
-    L.b200_profile_norm.argtypes = [vp, C.POINTER(C.c_int64)]
     L.b200_trace_decode.argtypes = [vp, i32, i32, vp, i32, C.POINTER(i32)]
     L.b200_tp_handle.argtypes = [vp, vp]
     L.b200_tp_attach.argtypes = [vp, vp, i32]
-    L.b200_test_seqsum.argtypes = [vp, i32, C.POINTER(C.c_float), C.POINTER(i32)]
     L.b200_set_prefill_mode.argtypes = [vp, i32]
     L.b200_set_decode_mode.argtypes = [vp, i32]
     L.b200_decode_info.argtypes = [vp, C.POINTER(i32), C.POINTER(i32), C.POINTER(i32), C.POINTER(i32)]
@@ -96,17 +94,14 @@ def _raise(code: int, msg: str):
     raise B200Error(code, msg)
 
 
-def test_seqsum(terms, want_info: bool = False, threads: int = 0):
-    """threads = 0: the round-1 accumulator (seqsum.cuh); 1024 / 256: seqsum2.cuh in the norm kernel's / persistent kernel's form."""
+def test_seqsum(terms, want_info: bool = False, threads: int = 1024):
+    """seqsum2.cuh run by threads = 1024 (the norm kernel's form), 512 (the persistent decode kernel's form) or 256."""
     t = np.ascontiguousarray(terms, dtype=np.float32)
     out = C.c_float(0)
     info = (C.c_int32 * 2)()
-    if threads:
-        rc = lib().b200_test_seqsum2(t.ctypes.data, len(t), threads, C.byref(out), info)
-    else:
-        rc = lib().b200_test_seqsum(t.ctypes.data, len(t), C.byref(out), info)
+    rc = lib().b200_test_seqsum2(t.ctypes.data, len(t), threads, C.byref(out), info)
     if rc != B200_OK:
-        _raise(rc, "b200_test_seqsum failed")
+        _raise(rc, "b200_test_seqsum2 failed")
     return (out.value, info[0], info[1]) if want_info else out.value
 
 
@@ -246,11 +241,6 @@ class NativePlan:
         n = C.c_int32(0)
         self._ck(lib().b200_trace_decode(self._p, token, position, rec.ctypes.data, cap, C.byref(n)))
         return rec[: n.value]
-
-    def profile_norm(self):
-        a = (C.c_int64 * 16)()
-        self._ck(lib().b200_profile_norm(self._p, a))
-        return list(a)
 
     def kv_reset(self):
         self._ck(lib().b200_kv_reset(self._p))

@@ -212,18 +212,10 @@ int b200_trace_decode(b200_plan *plan, int32_t token, int32_t position, uint64_t
  * {0 start, 1 final norm done, 2 lm_head rows done, 3 (CTA 0) step advanced}.  cap = capacity of stamps in uint64. */
 int b200_trace_persistent(b200_plan *plan, int32_t token, int32_t position, uint64_t *stamps, int64_t cap, int32_t *n_ctas, int32_t *n_rows, int32_t *n_stamps);
 
-/* Diagnostic: SM-clock cycles of the RMSNorm kernel's phases {launch->dependency wait, load+square,
- * exact sequential sum, normalise+quantise+store} followed by {entries, first fallback element or -1,
- * overflow flag} of the sequential-sum emulation, then at [8..12] the cycles of its phases
- * {group sums, head+prefix, group composition, barrier, resolve}.  cycles holds 16 int64. */
-int b200_profile_norm(b200_plan *plan, int64_t *cycles);
-
-/* Test hook for the exact parallel evaluation of the reference's sequential float sum
- * (csrc/seqsum.cuh; the RMSNorm accumulator of InferenceCore.java:39-48): sums n <= 8192
- * non-negative host floats on the device exactly as `for (i) s += t[i]` would. */
-int b200_test_seqsum(const float *terms, int32_t n, float *out, int32_t *info /* nullable: {entries, first fallback element or -1} */);
-/* Same contract for the round-2 accumulator (csrc/seqsum2.cuh) run by `threads` = 1024 (the RMSNorm kernel's form), 512
- * (the persistent decode kernel's form) or 256 threads; info = {items walked, fallbacks}. */
+/* Test hook for the exact parallel evaluation of the reference's sequential float sum (csrc/seqsum2.cuh; the RMSNorm
+ * accumulator of InferenceCore.java:39-48): sums n <= 8192 non-negative host floats on the device exactly as
+ * `for (i) s += t[i]` would, run by `threads` = 1024 (the RMSNorm kernel's form), 512 (the persistent decode kernel's form)
+ * or 256 threads; info = {items walked, fallbacks}. */
 int b200_test_seqsum2(const float *terms, int32_t n, int32_t threads, float *out, int32_t *info /* nullable */);
 
 /* Test hook for the device-side K-quant -> Q8_0 re-quantiser the upload pipeline applies to Q4_K / Q5_K / Q6_K tensors (csrc/kquant.cuh;
@@ -235,6 +227,10 @@ int b200_requant_kquant(int32_t ggml_type, const void *src, int64_t n_elems, voi
  * gemmMMA / gemmMMAQKV / gemmMMAGateUp, TransformerBatchPrefillKernels.java:792-1132) exposed for
  * tests and measurement: C[m][n] (f32) = A[m][k] (f16 bits) x B[n][k]^T (f16 bits) on tcgen05 tensor
  * cores, FP32 accumulation in TMEM.  Host pointers; m % 128 == n % 128 == k % 64 == 0.
+ * The kernel is one the prefill launches, chosen by B200_GEMM_2CTA / B200_GEMM_RESID / B200_GEMM_STAGES: 0 = single-CTA
+ * (C = A B^T, or C += A B^T with B200_GEMM_RESID=1; 3 or 6 stages), 256 = CTA-pair C += A B^T split B200_GEMM_RESID ways over k
+ * (needs B200_GEMM_RESID >= 1), 1256 = persistent CTA-pair C = A B^T (needs B200_GEMM_RESID unset or 0); CTA-pair kernels need
+ * m % 256 == n % 256 == 0.  Any other combination returns B200_ERR_BAD_ARG.
  * iters > 0 additionally times `iters` back-to-back launches (device events) into *ms. */
 int b200_gemm_f16(const uint16_t *a, const uint16_t *b, float *c, int32_t m, int32_t n, int32_t k, int32_t iters, float *ms /* nullable */);
 
@@ -242,7 +238,7 @@ int b200_gemm_f16(const uint16_t *a, const uint16_t *b, float *c, int32_t m, int
  * copy-in timing of TornadoVMMasterPlanSingleToken.java:51-54): wall seconds from the first tensor to the last repack kernel,
  * seconds the host spent copying mapped/pageable bytes into the pinned double buffer, and bytes sent over PCIe (a tensor-parallel
  * rank sends only its row ranges).  The pipeline: pinned double buffer filled by several host threads -> async H2D on a copy
- * stream -> double-buffered device staging -> repack kernel on the plan's stream; B200_UPLOAD_SYNC=1 selects blocking copies. */
+ * stream -> double-buffered device staging -> repack kernel on the plan's stream. */
 int b200_upload_info(b200_plan *plan, double *seconds, double *host_copy_seconds, int64_t *h2d_bytes);
 
 /* Number of kernels one decode step launches (bench.py's gpu_launches). */

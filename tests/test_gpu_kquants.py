@@ -73,15 +73,12 @@ def test_kquant_model_decodes_like_its_q8_0_twin(pkg, orc, shape, mix):
 
 
 def test_kquant_model_other_paths(pkg, orc, monkeypatch):
-    """The blocking upload (B200_UPLOAD_SYNC=1), the round-1 non-streaming kernels (B200_STREAM=0: every matrix goes through the
-    chunked split-plane upload) and the persistent decode kernel all see the same re-quantised weights."""
+    """The round-1 non-streaming kernels (B200_STREAM=0: every matrix goes through the chunked split-plane upload) and the
+    persistent decode kernel see the same re-quantised weights."""
     sh = pkg.synth.SHAPES["tiny-llama"]
     tensors = pkg.synth.build_tensors_kquant(sh, seed=12)
     m = pkg.loader.model_from_tensors(sh, pkg.gguf.GGMLType.Q8_0, tensors, 24)
     _decode_matches(pkg, orc, m, 6, mode="persistent")
-    monkeypatch.setenv("B200_UPLOAD_SYNC", "1")
-    _decode_matches(pkg, orc, m, 6)
-    monkeypatch.delenv("B200_UPLOAD_SYNC")
     monkeypatch.setenv("B200_STREAM", "0")
     _decode_matches(pkg, orc, m, 6)
 

@@ -326,10 +326,10 @@ def _seq(t):
     return np.add.accumulate(np.asarray(t, dtype=np.float32), dtype=np.float32)[-1]
 
 
-@pytest.mark.parametrize("threads", [0, 1024, 512, 256])
+@pytest.mark.parametrize("threads", [1024, 512, 256])
 def test_exact_parallel_sequential_sum(pkg, threads):
-    """csrc/seqsum.cuh (threads = 0) and csrc/seqsum2.cuh (1024 = the norm kernel's form, 512 = the persistent decode
-    kernel's form, 256 = a narrower one): the parallel emulation of `for (i) s += t[i]` in float32 must equal the
+    """csrc/seqsum2.cuh (1024 = the norm kernel's form, 512 = the persistent decode kernel's form, 256 = a narrower
+    one): the parallel emulation of `for (i) s += t[i]` in float32 must equal the
     literal chain bit for bit, on benign and adversarial inputs (ties, binade edges, zeros,
     huge dynamic range, sums parked next to a power of two, forced fallbacks)."""
     rng = np.random.default_rng(0)

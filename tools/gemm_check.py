@@ -17,10 +17,10 @@ out = []
 shapes = [(128, 128, 64), (256, 384, 512), (512, 4096, 4096)]
 if "--big" in sys.argv:
     shapes += [(512, 6144, 4096), (512, 28672, 4096), (512, 4096, 14336), (4096, 4096, 4096), (8192, 8192, 8192)]
+# 0: single-CTA kernel; 256: CTA-pair residual GEMM (needs B200_GEMM_RESID >= 1, the number of K splits); 1256: persistent pair kernel
 two = int(os.environ.get("B200_GEMM_2CTA", "0"))
 for (m, n, k) in shapes:
-    bn = 256 if two in (512, 1256) else two  # 512: two pair tiles per CTA pair; 1256: persistent pair kernel
-    if two and (m % (512 if two == 512 else 256) or n % bn):
+    if two and (m % 256 or n % 256):
         continue
     a = (rng.standard_normal((m, k)) * 0.5).astype(np.float16)
     b = (rng.standard_normal((n, k)) * 0.5).astype(np.float16)

@@ -5,8 +5,8 @@ reference's load-time metric, ModelLoader.java:102-106, and its first-execution 
     python tools/load_bench.py [workload] [dir]   ->  gpurun_out/load_bench_<workload>.json
 
 Writes a seeded synthetic GGUF of the real shape (no checkpoints offline), drops it from the process (the page cache may still hold it:
-reported as "warm"), then: parse + mmap (gguf.GGUFFile), b200_plan_create (pinned double buffer -> copy stream -> device staging ->
-repack kernels), and the same with the blocking round-1 path (B200_UPLOAD_SYNC=1)."""
+reported as "warm"), then: parse + mmap (gguf.GGUFFile) and b200_plan_create (pinned double buffer -> copy stream -> device staging ->
+repack kernels), with the default and with 8 host copy threads."""
 import json
 import os
 import sys
@@ -34,7 +34,7 @@ def main():
     size = os.path.getsize(path)
     del tensors, plan_order
     out = {"workload": workload, "file_bytes": size, "synthesise_s": gen_s, "write_s": write_s, "runs": []}
-    for label, env in (("pipelined", {}), ("blocking (round 1)", {"B200_UPLOAD_SYNC": "1"}), ("pipelined, 8 host threads", {"B200_UPLOAD_THREADS": "8"})):
+    for label, env in (("pipelined", {}), ("pipelined, 8 host threads", {"B200_UPLOAD_THREADS": "8"})):
         os.environ.update(env)
         try:
             t0 = time.time()

@@ -1,4 +1,4 @@
-"""Lane-accurate Python emulation of the segmented scan of csrc/experimental/seqsum2.cuh (seq2_warp_segscan, the scan over
+"""Lane-accurate Python emulation of the segmented scan of csrc/seqsum2.cuh (seq2_warp_segscan, the scan over
 the warp tails and the carry composition), checked against a sequential composition from each run's first thread.
 Pair composition is not commutative, so a wrong operand order or a wrong segment flag shows up immediately.
 usage: python tools/seqsum2/emulate_scan.py [cases]"""

@@ -1,5 +1,5 @@
 // harness.cu -- runs block_seqsum_exact_v2 (csrc/seqsum2.cuh) against the literal float loop on the
-// adversarial generators of proto.c and times it next to the round-1 kernel.
+// adversarial generators of proto.c and times it.
 // Build: nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -fmad=false -I gpullama3.java_b200/csrc -o /tmp/seqsum2_harness tools/seqsum2/harness.cu
 #include "seqsum2.cuh"
 #include <cmath>
@@ -29,15 +29,6 @@ __global__ void __launch_bounds__(256, 1) k_v2_256(const float *t, int n, float 
     const float s = block_seqsum_exact_v2_t<256>(sq, n, sc, (int)threadIdx.x, SeqSum2BlockSync());
     if (threadIdx.x == 0) { out[0] = s; info[0] = sc.info[0]; info[1] = sc.info[1]; }
 }
-__global__ void __launch_bounds__(SEQSUM_THREADS, 1) k_v1(const float *t, int n, float *out) {
-    extern __shared__ __align__(16) unsigned char sm1[];
-    float *sq = reinterpret_cast<float *>(sm1);
-    SeqSumScratch sc = seqsum_carve(sm1 + (size_t)n * 4, n);
-    for (int i = threadIdx.x; i < n; i += SEQSUM_THREADS) sq[i] = t[i];
-    __syncthreads();
-    const float s = block_seqsum_exact(sq, n, sc, nullptr);
-    if (threadIdx.x == 0) out[0] = s;
-}
 
 static unsigned long long rng = 88172645463325252ull;
 static unsigned xr() { rng ^= rng << 13; rng ^= rng >> 7; rng ^= rng << 17; return (unsigned)(rng >> 16); }
@@ -51,9 +42,8 @@ int main(int argc, char **argv) {
     int *dinfo;
     cudaMalloc(&dt, n * 4); cudaMalloc(&dout, 16); cudaMalloc(&dinfo, 16);
     const int E = (n + SEQSUM2_THREADS - 1) / SEQSUM2_THREADS;
-    const size_t smem2 = (size_t)SEQSUM2_THREADS * E * 4 + seqsum2_scratch_bytes(), smem1 = (size_t)n * 4 + seqsum_scratch_bytes(n);
+    const size_t smem2 = (size_t)SEQSUM2_THREADS * E * 4 + seqsum2_scratch_bytes();
     cudaFuncSetAttribute(k_v2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2);
-    cudaFuncSetAttribute(k_v1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1);
     const size_t smem3 = (size_t)256 * ((n + 255) / 256) * 4 + seqsum2_scratch_bytes();
     cudaFuncSetAttribute(k_v2_256, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem3);
     long bad = 0, items = 0, fb = 0;
@@ -94,17 +84,16 @@ int main(int argc, char **argv) {
     cudaEvent_t e0, e1;
     cudaEventCreate(&e0); cudaEventCreate(&e1);
     float ms;
-    for (int which = 0; which < 3; which++) {
+    for (int which = 0; which < 2; which++) {
         cudaEventRecord(e0);
         for (int r = 0; r < 200; r++) {
-            if (which == 2) k_v2_256<<<1, 256, smem3>>>(dt, n, dout, dinfo);
-            else if (which) k_v2<<<1, SEQSUM2_THREADS, smem2>>>(dt, n, dout, dinfo);
-            else k_v1<<<1, SEQSUM_THREADS, smem1>>>(dt, n, dout);
+            if (which) k_v2_256<<<1, 256, smem3>>>(dt, n, dout, dinfo);
+            else k_v2<<<1, SEQSUM2_THREADS, smem2>>>(dt, n, dout, dinfo);
         }
         cudaEventRecord(e1);
         cudaEventSynchronize(e1);
         cudaEventElapsedTime(&ms, e0, e1);
-        printf("%s: %.2f us per launch (back-to-back launches, includes ~2 us launch overhead)\n", which == 2 ? "v2 (256 threads)" : which ? "v2" : "v1", ms * 1000.f / 200);
+        printf("%s: %.2f us per launch (back-to-back launches, includes ~2 us launch overhead)\n", which ? "v2 (256 threads)" : "v2", ms * 1000.f / 200);
     }
     return bad != 0;
 }

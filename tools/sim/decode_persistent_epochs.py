@@ -1,4 +1,4 @@
-"""Model of the grid-wide phase synchronisation of k_decode_persistent (csrc/experimental/decode_persistent.cuh): monotone epoch
+"""Model of the grid-wide phase synchronisation of k_decode_persistent (csrc/decode_persistent.cuh): monotone epoch
 counters with the kernel's exact target expressions, several CTAs, several layers, several launches (decode launches with
 lm_head and prefill launches without), random interleavings.  Checks: no deadlock; a phase never starts before every
 producer of its input finished (all QKV rows before attention, all heads before Wo, all rows of x before a norm, the whole
