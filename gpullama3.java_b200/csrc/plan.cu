@@ -54,6 +54,12 @@ struct Uploader {
     int64_t h2d_bytes = 0;
 };
 
+// The kernels every decode matvec of a plan runs on, chosen once in build() from the weight type and the shapes:
+// the Q8_0 tile stream (k_stream_matvec_q8), the Q8_0 row kernels (k_matvec_q8, k_gateup_q8), the FP16 per-warp rings
+// (k_stream_matvec_f16) or the FP16 row kernels (k_matvec_f16, k_swiglu).  The row kernels serve the shapes the other
+// two layouts do not fit.
+enum MvPath { Q8_TILES, Q8_ROWS, F16_RINGS, F16_ROWS };
+
 struct b200_plan {
     b200_config cfg{};
     Uploader up;
@@ -68,10 +74,11 @@ struct b200_plan {
 
     DevMat emb{}, out{};
     TileMat tout{};
-    bool use_stream = false, use_pdl = false;
+    MvPath path = Q8_ROWS;
+    // The tile stream and the rings launch with PDL, leave per-CTA argmax partials of the classifier and stamp trace records.
+    bool streaming() const { return path == Q8_TILES || path == F16_RINGS; }
     int kflags = 0; // KF_* (common.cuh): what the attention prologues do for this architecture
     size_t kq_off = 0; // K-quant files: offset of the raw (K-quant bytes) area inside each staging buffer; 0 = no K-quant tensor in the file
-    bool use_f16_stream = false; // FP16 plans: per-warp bulk-copy rings (stream_matvec_f16.cuh) instead of k_matvec_f16
     bool f16_copies = false; // Q8_0 plan that also holds f16 weight matrices for the tensor-core prefill
     int n_sms = 148;
     unsigned *blk_cnt = nullptr;
@@ -179,8 +186,6 @@ void par_memcpy(void *dst, const void *src, size_t n, int threads) {
 
 int up_init(b200_plan *p, size_t dst_bytes) {
     Uploader &u = p->up;
-    const char *t = getenv("B200_UPLOAD_THREADS");
-    u.threads = t ? atoi(t) : 4;
     u.pin_bytes = (size_t)64 << 20;
     u.dst_bytes = dst_bytes;
     CK(cudaStreamCreateWithFlags(&u.copy, cudaStreamNonBlocking));
@@ -457,7 +462,7 @@ int sf_grid(const b200_plan *p, int rows, int cols, bool gateup) { // CTAs of an
     const int grid = L.ctas_per_sm * p->n_sms;
     return grid > rows / mr ? rows / mr : grid;
 }
-template <int MODE> int launch_stream_f16(b200_plan *p, const DevMat &m, const DevMat *m2, const float *x, float *out, TraceBuf tr = TraceBuf{nullptr, 0, 0},
+template <int MODE> int launch_stream_f16(b200_plan *p, bool pdl, const DevMat &m, const DevMat *m2, const float *x, float *out, TraceBuf tr,
                                           bool argmax = false) {
     const int lanes = p->cfg.fp16_lanes;
     const SfLayout L = sf_layout(m.rows, m.cols, lanes, MODE == SF_GATEUP);
@@ -468,8 +473,8 @@ template <int MODE> int launch_stream_f16(b200_plan *p, const DevMat &m, const D
     a.part_val = argmax ? p->part_val : nullptr;
     a.part_idx = argmax ? p->part_idx : nullptr;
     const int grid = sf_grid(p, m.rows, m.cols, MODE == SF_GATEUP);
-    if (lanes == 16) return launch_k(p, p->use_pdl, k_stream_matvec_f16<16, MODE>, dim3(grid), dim3(SF_THREADS), L.total, a);
-    return launch_k(p, p->use_pdl, k_stream_matvec_f16<8, MODE>, dim3(grid), dim3(SF_THREADS), L.total, a);
+    if (lanes == 16) return launch_k(p, pdl, k_stream_matvec_f16<16, MODE>, dim3(grid), dim3(SF_THREADS), L.total, a);
+    return launch_k(p, pdl, k_stream_matvec_f16<8, MODE>, dim3(grid), dim3(SF_THREADS), L.total, a);
 }
 
 // Kernel launch with the programmatic-dependent-launch attribute (captured into the CUDA graph as
@@ -497,12 +502,13 @@ void read_knobs(b200_plan *p) {
     // default: the CUDA graph -- measured faster than the persistent kernel on the same box (profiles/r2_final_a.log: 313.6 vs 285.1 tok/s,
     // 8B Q8_0; under tensor parallelism by 10-21 %).  B200_DECODE=persistent or b200_set_decode_mode select the one-kernel-per-token path.
     p->decode_mode = (d && !strcmp(d, "persistent")) ? B200_DECODE_PERSISTENT : B200_DECODE_GRAPH;
+    const char *t = getenv("B200_UPLOAD_THREADS"); // host threads filling the pinned upload buffers
+    if (t) p->up.threads = atoi(t);
 }
 
 template <int MODE>
-int launch_stream(b200_plan *p, const TileMat &W, const int8_t *xq, const float *xs, float *out, int8_t *hq, float *hs, bool argmax = false,
-                  TraceBuf tr = TraceBuf{nullptr, 0, 0}, int wait_slot = -1, unsigned wait_op = 0, int out_slot = -1, unsigned out_op = 0,
-                  int row_base = 0) {
+int launch_stream(b200_plan *p, bool pdl, const TileMat &W, const int8_t *xq, const float *xs, float *out, int8_t *hq, float *hs, bool argmax,
+                  TraceBuf tr, int wait_slot = -1, unsigned wait_op = 0, int out_slot = -1, unsigned out_op = 0, int row_base = 0) {
     SmvSmem L = smv_layout(W.cols, W.seg, SMV_SMEM_BUDGET_MAX);
     SmvArgs a;
     a.W = W; a.xq = xq; a.xs = xs; a.out = out; a.hq = hq; a.hs = hs; a.blk_cnt = p->blk_cnt;
@@ -511,7 +517,7 @@ int launch_stream(b200_plan *p, const TileMat &W, const int8_t *xq, const float 
     a.tr = tr;
     a.tp = p->tp;
     a.wait_slot = wait_slot; a.wait_op = wait_op; a.out_slot = out_slot; a.out_op = out_op; a.row_base = row_base;
-    return launch_k(p, p->use_pdl, k_stream_matvec_q8<MODE>, dim3(p->n_sms), dim3(SMV_THREADS), L.total, a, L);
+    return launch_k(p, pdl, k_stream_matvec_q8<MODE>, dim3(p->n_sms), dim3(SMV_THREADS), L.total, a, L);
 }
 
 bool stream_shape_ok(int rows, int cols) {
@@ -528,13 +534,69 @@ bool gateup_fits(int hidden, int n_sms) { // epilogue buffer holds this CTA's hi
 // k_attention's dynamic shared memory: q | k | out | score row (the row lives in a global scratch buffer for long contexts).
 size_t att_smem_bytes(int head_size, int ctx, bool scratch) { return (size_t)(3 * head_size + (scratch ? 0 : ctx)) * 4; }
 
+// The matrix roles of a decode step; the values are b200_time_kernel's kernel ids.
+enum MvRole { MV_GATEUP, MV_W2, MV_QKV, MV_WO, MV_CLS };
+
+// Launches matrix role `role` of layer l (the classifier ignores l) on the plan's path; returns how many kernels it launched,
+// or a negative B200_ERR_*.  Under tensor parallelism a forward numbers its flag epochs op = 4*l + {0: attention out,
+// 1: x after Wo, 2: hb, 3: x after W2}: the tile stream waits on the slot that carries its activation and publishes its output.
+int launch_mv(b200_plan *p, MvRole role, int l, bool pdl, TraceBuf tr) {
+    const b200_config &c = p->cfg;
+    LayerW &L = p->layers[l];
+    int rc = B200_OK, n = 1;
+    if (p->path == Q8_TILES) {
+        const bool tpar = p->tp.n > 1;
+        const int slot_att = tpar ? TP_SLOT_ATT : -1, slot_x = tpar ? TP_SLOT_X : -1, slot_hq = tpar ? TP_SLOT_HQ : -1, rank = p->tp.rank;
+        const unsigned op = 4u * l;
+        switch (role) {
+        case MV_QKV: rc = launch_stream<SMV_STORE>(p, pdl, L.tqkv, p->xq, p->xs, p->qkv, nullptr, nullptr, false, tr); break;
+        case MV_WO: rc = launch_stream<SMV_RESID>(p, pdl, L.two, p->attq, p->atts, p->x, nullptr, nullptr, false, tr, slot_att, op + 0, slot_x, op + 1, rank * p->dim_l); break;
+        case MV_GATEUP: rc = launch_stream<SMV_GATEUP>(p, pdl, L.tgu, p->xq, p->xs, p->hb, p->hq, p->hs, false, tr, -1, 0, slot_hq, op + 2, rank * p->hid_l); break;
+        case MV_W2: rc = launch_stream<SMV_RESID>(p, pdl, L.tw2, p->hq, p->hs, p->x, nullptr, nullptr, false, tr, slot_hq, op + 2, slot_x, op + 3, rank * p->dim_l); break;
+        case MV_CLS: rc = launch_stream<SMV_STORE>(p, pdl, p->tout, p->xq, p->xs, p->logits, nullptr, nullptr, true, tr, -1, 0, -1, 0, rank * p->voc_l); break;
+        }
+    } else if (p->path == Q8_ROWS) {
+        switch (role) {
+        case MV_QKV: rc = launch_matvec_q8<MODE_STORE>(p, L.qkv, p->xq, p->xs, p->qkv); break;
+        case MV_WO: rc = launch_matvec_q8<MODE_RESID>(p, L.wo, p->xq, p->xs, p->x); break;
+        case MV_GATEUP:
+            k_gateup_q8<<<c.hidden_dim / 32, 256, q8_smem_bytes(c.dim, 4, 8), p->stream>>>(
+                (const int8_t *)L.w1.qs, L.w1.sc, (const int8_t *)L.w3.qs, L.w3.sc, p->xq, p->xs, c.hidden_dim, c.dim, p->hq, p->hs, p->hb);
+            CK(cudaGetLastError());
+            break;
+        case MV_W2: rc = launch_matvec_q8<MODE_RESID>(p, L.w2, p->hq, p->hs, p->x); break;
+        case MV_CLS: rc = launch_matvec_q8<MODE_STORE>(p, p->out, p->xq, p->xs, p->logits); break;
+        }
+    } else if (p->path == F16_RINGS) {
+        switch (role) {
+        case MV_QKV: rc = launch_stream_f16<SF_STORE>(p, pdl, L.qkv, nullptr, p->xb, p->qkv, tr); break;
+        case MV_WO: rc = launch_stream_f16<SF_RESID>(p, pdl, L.wo, nullptr, p->xb, p->x, tr); break;
+        case MV_GATEUP: rc = launch_stream_f16<SF_GATEUP>(p, pdl, L.w1, &L.w3, p->xb, p->hb, tr); break; // gate, up and SwiGLU in one launch
+        case MV_W2: rc = launch_stream_f16<SF_RESID>(p, pdl, L.w2, nullptr, p->hb, p->x, tr); break;
+        case MV_CLS: rc = launch_stream_f16<SF_STORE>(p, pdl, p->out, nullptr, p->xb, p->logits, tr, true); break;
+        }
+    } else {
+        switch (role) {
+        case MV_QKV: rc = launch_matvec_f16<MODE_STORE>(p, L.qkv, p->xb, p->qkv); break;
+        case MV_WO: rc = launch_matvec_f16<MODE_RESID>(p, L.wo, p->xb, p->x); break;
+        case MV_GATEUP:
+            if ((rc = launch_matvec_f16<MODE_STORE>(p, L.w1, p->xb, p->hb)) || (rc = launch_matvec_f16<MODE_STORE>(p, L.w3, p->xb, p->hb2))) break;
+            k_swiglu<<<(c.hidden_dim + 255) / 256, 256, 0, p->stream>>>(p->hb, p->hb2, c.hidden_dim);
+            CK(cudaGetLastError());
+            n = 3;
+            break;
+        case MV_W2: rc = launch_matvec_f16<MODE_RESID>(p, L.w2, p->hb, p->x); break;
+        case MV_CLS: rc = launch_matvec_f16<MODE_STORE>(p, p->out, p->xb, p->logits); break;
+        }
+    }
+    return rc ? rc : n;
+}
+
 // Enqueue one single-token forward on p->stream (captured into a CUDA graph at creation).
 // with_logits=false is the prefill variant (InferenceCoreBatchPrefillDecode.java:166-167).
 int enqueue_forward(b200_plan *p, bool with_logits, int *launches, bool trace = false) {
     const b200_config &c = p->cfg;
-    const bool q8 = p->wtype == B200_GGML_Q8_0;
-    const bool st = p->use_stream, pdl = p->use_pdl, sf = p->use_f16_stream;
-    const bool tpar = p->tp.n > 1;
+    const bool q8 = p->wtype == B200_GGML_Q8_0, pdl = p->streaming();
     int n = 0;
     auto TR = [&](int id) { return TraceBuf{trace ? p->trace_rec : nullptr, n, id}; };
     const size_t norm_smem = norm_smem_bytes(c.dim);
@@ -552,14 +614,11 @@ int enqueue_forward(b200_plan *p, bool with_logits, int *launches, bool trace = 
     for (int l = 0; l < c.n_layers; l++) {
         LayerW &L = p->layers[l];
         int rc;
-        // TP flag epochs inside one forward: op = 4*l + {0: attention out, 1: x after Wo, 2: hb, 3: x after W2}
+        // TP flag epochs: see launch_mv
         if ((rc = norm(l == 0, L.attn_norm, l == 0 ? -1 : 4 * (l - 1) + 3))) return rc;
         n++;
-        if (st) rc = launch_stream<SMV_STORE>(p, L.tqkv, p->xq, p->xs, p->qkv, nullptr, nullptr, false, TR(2));
-        else if (q8) rc = launch_matvec_q8<MODE_STORE>(p, L.qkv, p->xq, p->xs, p->qkv);
-        else if (sf) rc = launch_stream_f16<SF_STORE>(p, L.qkv, nullptr, p->xb, p->qkv, TR(2));
-        else rc = launch_matvec_f16<MODE_STORE>(p, L.qkv, p->xb, p->qkv);
-        if (rc) return rc; n++;
+        if ((rc = launch_mv(p, MV_QKV, l, pdl, TR(2))) < 0) return rc;
+        n += rc;
         float *kc = p->key_cache + (size_t)l * ctx_kv, *vc = p->value_cache + (size_t)l * ctx_kv;
         {
             const size_t att_smem = att_smem_bytes(c.head_size, c.context_length, p->att_scratch != nullptr);
@@ -577,31 +636,14 @@ int enqueue_forward(b200_plan *p, bool with_logits, int *launches, bool trace = 
             if (rc) return rc;
             n++;
         }
-        if (st) rc = launch_stream<SMV_RESID>(p, L.two, p->attq, p->atts, p->x, nullptr, nullptr, false, TR(5), tpar ? TP_SLOT_ATT : -1, 4 * l + 0, tpar ? TP_SLOT_X : -1, 4 * l + 1, rank * p->dim_l);
-        else if (q8) rc = launch_matvec_q8<MODE_RESID>(p, L.wo, p->xq, p->xs, p->x);
-        else if (sf) rc = launch_stream_f16<SF_RESID>(p, L.wo, nullptr, p->xb, p->x, TR(5));
-        else rc = launch_matvec_f16<MODE_RESID>(p, L.wo, p->xb, p->x);
-        if (rc) return rc; n++;
+        if ((rc = launch_mv(p, MV_WO, l, pdl, TR(5))) < 0) return rc;
+        n += rc;
         if ((rc = norm(false, L.ffn_norm, 4 * l + 1))) return rc;
         n++;
-        if (st) {
-            if ((rc = launch_stream<SMV_GATEUP>(p, L.tgu, p->xq, p->xs, p->hb, p->hq, p->hs, false, TR(6), -1, 0, tpar ? TP_SLOT_HQ : -1, 4 * l + 2, rank * p->hid_l))) return rc; n++;
-            if ((rc = launch_stream<SMV_RESID>(p, L.tw2, p->hq, p->hs, p->x, nullptr, nullptr, false, TR(7), tpar ? TP_SLOT_HQ : -1, 4 * l + 2, tpar ? TP_SLOT_X : -1, 4 * l + 3, rank * p->dim_l))) return rc; n++;
-        } else if (q8) {
-            k_gateup_q8<<<c.hidden_dim / 32, 256, q8_smem_bytes(c.dim, 4, 8), p->stream>>>(
-                (const int8_t *)L.w1.qs, L.w1.sc, (const int8_t *)L.w3.qs, L.w3.sc, p->xq, p->xs, c.hidden_dim, c.dim, p->hq, p->hs, p->hb);
-            CK(cudaGetLastError()); n++;
-            if ((rc = launch_matvec_q8<MODE_RESID>(p, L.w2, p->hq, p->hs, p->x))) return rc; n++;
-        } else if (sf) { // gate, up and SwiGLU in one launch; then the down projection
-            if ((rc = launch_stream_f16<SF_GATEUP>(p, L.w1, &L.w3, p->xb, p->hb, TR(6)))) return rc; n++;
-            if ((rc = launch_stream_f16<SF_RESID>(p, L.w2, nullptr, p->hb, p->x, TR(7)))) return rc; n++;
-        } else {
-            if ((rc = launch_matvec_f16<MODE_STORE>(p, L.w1, p->xb, p->hb))) return rc; n++;
-            if ((rc = launch_matvec_f16<MODE_STORE>(p, L.w3, p->xb, p->hb2))) return rc; n++;
-            k_swiglu<<<(c.hidden_dim + 255) / 256, 256, 0, p->stream>>>(p->hb, p->hb2, c.hidden_dim);
-            CK(cudaGetLastError()); n++;
-            if ((rc = launch_matvec_f16<MODE_RESID>(p, L.w2, p->hb, p->x))) return rc; n++;
-        }
+        if ((rc = launch_mv(p, MV_GATEUP, l, pdl, TR(6))) < 0) return rc;
+        n += rc;
+        if ((rc = launch_mv(p, MV_W2, l, pdl, TR(7))) < 0) return rc;
+        n += rc;
     }
     const int last_x_op = 4 * (c.n_layers - 1) + 3;
     if (with_logits) {
@@ -609,17 +651,15 @@ int enqueue_forward(b200_plan *p, bool with_logits, int *launches, bool trace = 
         int rc;
         if ((rc = norm(false, p->out_norm, last_x_op))) return rc;
         n++;
-        if (st) rc = launch_stream<SMV_STORE>(p, p->tout, p->xq, p->xs, p->logits, nullptr, nullptr, true, TR(8), -1, 0, -1, 0, rank * p->voc_l);
-        else if (q8) rc = launch_matvec_q8<MODE_STORE>(p, p->out, p->xq, p->xs, p->logits);
-        else if (sf) rc = launch_stream_f16<SF_STORE>(p, p->out, nullptr, p->xb, p->logits, TR(8), true);
-        else rc = launch_matvec_f16<MODE_STORE>(p, p->out, p->xb, p->logits);
-        if (rc) return rc; n++;
+        if ((rc = launch_mv(p, MV_CLS, 0, pdl, TR(8))) < 0) return rc;
+        n += rc;
     }
     {
         int rc;
+        // part_val / part_idx exist only on the streaming paths; the row kernels leave the whole argmax to this kernel
         if ((rc = launch_k(p, pdl, k_argmax_advance, dim3(1), dim3(1024), (size_t)0, (const float *)p->logits, c.vocab_size, p->st, (const int *)p->seq_tokens, p->out_ids, with_logits ? 1 : 0,
-                           (const float *)(st || sf ? p->part_val : nullptr), (const int *)(st || sf ? p->part_idx : nullptr),
-                           sf ? sf_grid(p, c.vocab_size, c.dim, false) : p->n_sms, TR(9), p->tp, with_logits ? -1 : last_x_op))) return rc;
+                           (const float *)p->part_val, (const int *)p->part_idx, p->path == F16_RINGS ? sf_grid(p, c.vocab_size, c.dim, false) : p->n_sms,
+                           TR(9), p->tp, with_logits ? -1 : last_x_op))) return rc;
         n++;
     }
     if (launches) *launches = n;
@@ -632,7 +672,7 @@ int enqueue_forward(b200_plan *p, bool with_logits, int *launches, bool trace = 
 int pd_prepare(b200_plan *p) {
     const b200_config &c = p->cfg;
     p->pd_ok = false;
-    if (!p->use_stream) { p->pd_why = "the persistent decode kernel needs the Q8_0 streaming layout"; return B200_OK; }
+    if (p->path != Q8_TILES) { p->pd_why = "the persistent decode kernel needs the Q8_0 streaming layout"; return B200_OK; }
     if (c.head_size != 64 && c.head_size != 128) { p->pd_why = "the persistent decode kernel supports head sizes 64 and 128"; return B200_OK; }
     if (p->nh_l > p->n_sms) { p->pd_why = "more attention heads than SMs"; return B200_OK; }
     if (!gateup_fits(p->hid_l, p->n_sms)) { p->pd_why = "hidden slice per CTA exceeds the epilogue buffer"; return B200_OK; }
@@ -721,7 +761,7 @@ int capture_all(b200_plan *p) {
     int rc;
     if ((rc = capture(p, true, &p->g_decode, &p->launches_decode))) return rc;
     if ((rc = capture(p, false, &p->g_prefill, nullptr))) return rc;
-    if (p->use_stream || p->use_f16_stream) {
+    if (p->streaming()) {
         if ((rc = dalloc(p, &p->trace_rec, (size_t)(p->launches_decode + 8) * 32))) return rc;
         if ((rc = capture(p, true, &p->g_trace, nullptr, true))) return rc;
     }
@@ -730,7 +770,7 @@ int capture_all(b200_plan *p) {
         // grid = one CTA per SM with (almost) all of its shared memory: co-resident on an idle GPU either way; the cooperative
         // attribute makes the driver check it.  Should a driver refuse cooperative kernel nodes in a graph, retry without.
         for (int attempt = 0; attempt < 2; attempt++) {
-            p->pd_coop = attempt == 0 && !getenv("B200_PD_NO_COOP");
+            p->pd_coop = attempt == 0;
             rc = capture(p, true, &p->g_pdecode, nullptr, false, true);
             if (!rc) rc = capture(p, false, &p->g_pprefill, nullptr, false, true);
             if (!rc) rc = capture(p, true, &p->g_ptrace, nullptr, true, true);
@@ -837,22 +877,19 @@ int build(b200_plan *p, const b200_tensor *tensors, int n_tensors) {
     CK(cudaEventCreate(&p->ev1));
     int rc;
     CK(cudaDeviceGetAttribute(&p->n_sms, cudaDevAttrMultiProcessorCount, p->device));
-    {
-        const char *e = getenv("B200_STREAM");
-        bool want = !(e && e[0] == '0');
-        p->use_stream = want && p->wtype == B200_GGML_Q8_0 && stream_shape_ok(p->qd_l + 2 * p->kvd_l, c.dim) && stream_shape_ok(p->dim_l, p->qd) &&
-                        stream_shape_ok(2 * p->hid_l, c.dim) && stream_shape_ok(p->dim_l, c.hidden_dim) && stream_shape_ok(p->voc_l, c.dim) &&
-                        gateup_fits(p->hid_l, p->n_sms);
-        const char *e3 = getenv("B200_F16_STREAM"); // FP16 plans: 0 = the round-1 k_matvec_f16 launches
-        p->use_f16_stream = !(e3 && e3[0] == '0') && p->wtype == B200_GGML_F16 && c.tp_size == 1 && sf_layout(p->qd + 2 * p->kvd, c.dim, c.fp16_lanes, false).ok &&
-                            sf_layout(c.dim, p->qd, c.fp16_lanes, false).ok && sf_layout(c.hidden_dim, c.dim, c.fp16_lanes, true).ok &&
-                            sf_layout(c.dim, c.hidden_dim, c.fp16_lanes, false).ok && sf_layout(c.vocab_size, c.dim, c.fp16_lanes, false).ok;
-        const char *e2 = getenv("B200_PDL");
-        p->use_pdl = (p->use_stream || p->use_f16_stream) && !(e2 && e2[0] == '0');
-        if (c.tp_size > 1 && !p->use_stream) return fail(p, B200_ERR_UNSUPPORTED, "tensor parallelism needs the Q8_0 streaming path");
+    if (p->wtype == B200_GGML_Q8_0) {
+        const bool tiles = stream_shape_ok(p->qd_l + 2 * p->kvd_l, c.dim) && stream_shape_ok(p->dim_l, p->qd) && stream_shape_ok(2 * p->hid_l, c.dim) &&
+                           stream_shape_ok(p->dim_l, c.hidden_dim) && stream_shape_ok(p->voc_l, c.dim) && gateup_fits(p->hid_l, p->n_sms);
+        p->path = tiles ? Q8_TILES : Q8_ROWS;
+    } else {
+        const int lanes = c.fp16_lanes;
+        const bool rings = sf_layout(p->qd + 2 * p->kvd, c.dim, lanes, false).ok && sf_layout(c.dim, p->qd, lanes, false).ok &&
+                           sf_layout(c.hidden_dim, c.dim, lanes, true).ok && sf_layout(c.dim, c.hidden_dim, lanes, false).ok && sf_layout(c.vocab_size, c.dim, lanes, false).ok;
+        p->path = rings ? F16_RINGS : F16_ROWS;
     }
+    if (c.tp_size > 1 && p->path != Q8_TILES) return fail(p, B200_ERR_UNSUPPORTED, "tensor parallelism needs the Q8_0 streaming path");
     size_t stage_bytes = (size_t)34 * (8u << 20); // 8 Mi blocks = 272 MiB
-    if (p->use_stream) {
+    if (p->path == Q8_TILES) {
         size_t m1 = (size_t)c.vocab_size * c.dim, m2 = (size_t)2 * c.hidden_dim * c.dim, m3 = (size_t)(p->qd + 2 * p->kvd) * c.dim;
         size_t mx = m1 > m2 ? m1 : m2;
         if (m3 > mx) mx = m3;
@@ -872,31 +909,21 @@ int build(b200_plan *p, const b200_tensor *tensors, int n_tensors) {
     if ((rc = alloc_matrix(p, p->emb, c.vocab_size, c.dim, eff_type(emb->ggml_type)))) return rc;
     if ((rc = upload_matrix(p, emb, c.vocab_size, c.dim, p->emb, 0))) return rc;
     const b200_tensor *outw = find(tensors, n_tensors, "output.weight");
-    if (p->use_stream) {
-        if (!outw && eff_type(emb->ggml_type) != p->wtype) return fail(p, B200_ERR_UNSUPPORTED, "tied output weight type differs from the matrix type");
-        {
-            const int r0[3] = {c.tp_rank * p->voc_l, 0, 0}, fu[3] = {c.vocab_size, 0, 0};
-            if ((rc = upload_tiles(p, outw ? outw : emb, nullptr, nullptr, p->voc_l, 0, 0, c.dim, false, p->tout, r0, fu))) return rc;
-        }
-        p->out = p->emb;
-        if ((rc = dalloc(p, &p->part_val, (size_t)p->n_sms * 4))) return rc;
-        if ((rc = dalloc(p, &p->part_idx, (size_t)p->n_sms * 4))) return rc;
+    if (!outw && eff_type(emb->ggml_type) != p->wtype) return fail(p, B200_ERR_UNSUPPORTED, "tied output weight type differs from the matrix type");
+    p->out = p->emb; // a tied classifier; replaced below when the file has its own and the row kernels or rings read it
+    if (p->path == Q8_TILES) {
+        const int r0[3] = {c.tp_rank * p->voc_l, 0, 0}, fu[3] = {c.vocab_size, 0, 0};
+        if ((rc = upload_tiles(p, outw ? outw : emb, nullptr, nullptr, p->voc_l, 0, 0, c.dim, false, p->tout, r0, fu))) return rc;
         if ((rc = dalloc(p, &p->blk_cnt, (size_t)(c.hidden_dim / 32) * 4))) return rc;
         CK(cudaMemset(p->blk_cnt, 0, (size_t)(c.hidden_dim / 32) * 4));
     } else if (outw) {
-        if (p->use_f16_stream) { // per-CTA argmax partials of the classifier launch (at most 3 CTAs per SM)
-            if ((rc = dalloc(p, &p->part_val, (size_t)p->n_sms * 4 * 4))) return rc;
-            if ((rc = dalloc(p, &p->part_idx, (size_t)p->n_sms * 4 * 4))) return rc;
-        }
         if ((rc = alloc_matrix(p, p->out, c.vocab_size, c.dim, p->wtype))) return rc;
         if ((rc = upload_matrix(p, outw, c.vocab_size, c.dim, p->out, 0))) return rc;
-    } else {
-        if (eff_type(emb->ggml_type) != p->wtype) return fail(p, B200_ERR_UNSUPPORTED, "tied output weight type differs from the matrix type");
-        p->out = p->emb;
-        if (p->use_f16_stream) {
-            if ((rc = dalloc(p, &p->part_val, (size_t)p->n_sms * 4 * 4))) return rc;
-            if ((rc = dalloc(p, &p->part_idx, (size_t)p->n_sms * 4 * 4))) return rc;
-        }
+    }
+    if (p->streaming()) { // per-CTA argmax partials of the classifier launch: one CTA per SM on the tile stream, at most 3 on the rings
+        const size_t parts = (size_t)p->n_sms * (p->path == F16_RINGS ? 4 : 1);
+        if ((rc = dalloc(p, &p->part_val, parts * 4))) return rc;
+        if ((rc = dalloc(p, &p->part_idx, parts * 4))) return rc;
     }
     if ((rc = upload_f32(p, find(tensors, n_tensors, "output_norm.weight"), c.dim, &p->out_norm, "output_norm.weight"))) return rc;
 
@@ -919,7 +946,7 @@ int build(b200_plan *p, const b200_tensor *tensors, int n_tensors) {
         const b200_tensor *tg = T(phi3 ? "ffn_up.weight" : "ffn_gate.weight"), *tu = T("ffn_up.weight");
         const int q_full = phi3 ? p->qd + 2 * p->kvd : p->qd, k_full = phi3 ? q_full : p->kvd, g_full = phi3 ? 2 * c.hidden_dim : c.hidden_dim;
         const int k_src = phi3 ? p->qd : 0, v_src = phi3 ? p->qd + p->kvd : 0, u_src = phi3 ? c.hidden_dim : 0;
-        if (p->use_stream) {
+        if (p->path == Q8_TILES) {
             const int rk = c.tp_rank;
             const int qr0[3] = {rk * p->qd_l, k_src + rk * p->kvd_l, v_src + rk * p->kvd_l}, qfu[3] = {q_full, k_full, k_full};
             if ((rc = upload_tiles(p, tq, tk, tv, p->qd_l, p->kvd_l, p->kvd_l, c.dim, false, L.tqkv, qr0, qfu))) return rc;
@@ -1056,8 +1083,8 @@ int prefill_init(b200_plan *p) {
     c.mode = 0;
     const int kv_mul = g.n_heads / g.n_kv_heads, nqkv = p->qd + 2 * p->kvd;
     if (p->wtype != B200_GGML_F16 && !p->f16_copies) {
-        c.why = p->use_stream ? "Q8_0 plan: the tensor-core prefill is opt-in (b200_set_prefill_mode builds f16 twins of the weight matrices, +2 bytes per weight)"
-                              : "tensor-core prefill needs FP16 weight matrices or a Q8_0 plan on the streaming path";
+        c.why = p->path == Q8_TILES ? "Q8_0 plan: the tensor-core prefill is opt-in (b200_set_prefill_mode builds f16 twins of the weight matrices, +2 bytes per weight)"
+                                    : "tensor-core prefill needs FP16 weight matrices or a Q8_0 plan on the streaming path";
         return B200_OK;
     }
     if (g.tp_size > 1) { c.why = "tensor-core prefill is single-GPU"; return B200_OK; }
@@ -1084,18 +1111,15 @@ int prefill_init(b200_plan *p) {
     bool ok = pg::make_map(&c.mA, c.A16, c.bpad, g.dim, pg::BM) == 0 && pg::make_map(&c.mATT, c.ATT16, c.bpad, p->qd, pg::BM) == 0 &&
               pg::make_map(&c.mH, c.H16, c.bpad, g.hidden_dim, pg::BM) == 0 && pg::make_map_c(&c.mX, c.X, c.bpad, g.dim) == 0 &&
               pg::make_map_c(&c.mQKV, c.QKV, c.bpad, nqkv) == 0;
+    c.pair = nqkv % 256 == 0 && g.dim % 256 == 0 && g.hidden_dim % 128 == 0; // the GEMMs divide into 256-wide pair tiles
+    const int gu_box = c.pair ? 128 : pg::BN / 2; // gate/up tile: 128 + 128 weight rows on a CTA pair, 64 + 64 on one CTA
     c.maps.resize(g.n_layers);
     for (int l = 0; ok && l < g.n_layers; l++) {
         const LayerW &L = p->layers[l];
         PrefillLayerMaps &m = c.maps[l];
         ok = pg::make_map(&m.qkv, L.qkv.qs, nqkv, g.dim, pg::BN) == 0 && pg::make_map(&m.wo, L.wo.qs, g.dim, p->qd, pg::BN) == 0 &&
-             pg::make_map(&m.w1, L.w1.qs, g.hidden_dim, g.dim, pg::BN / 2) == 0 && pg::make_map(&m.w3, L.w3.qs, g.hidden_dim, g.dim, pg::BN / 2) == 0 &&
-             pg::make_map(&m.w2, L.w2.qs, g.dim, g.hidden_dim, pg::BN) == 0 && pg::make_map(&m.w1p, L.w1.qs, g.hidden_dim, g.dim, 128) == 0 &&
-             pg::make_map(&m.w3p, L.w3.qs, g.hidden_dim, g.dim, 128) == 0;
-    }
-    {
-        const char *e = getenv("B200_GEMM_2CTA");
-        c.pair = !(e && e[0] == '0') && nqkv % 256 == 0 && g.dim % 256 == 0 && g.hidden_dim % 128 == 0;
+             pg::make_map(&m.w1, L.w1.qs, g.hidden_dim, g.dim, gu_box) == 0 && pg::make_map(&m.w3, L.w3.qs, g.hidden_dim, g.dim, gu_box) == 0 &&
+             pg::make_map(&m.w2, L.w2.qs, g.dim, g.hidden_dim, pg::BN) == 0;
     }
     if (!ok) { c.why = "cuTensorMapEncodeTiled rejected a tensor map"; return B200_OK; }
     if (g.head_size == 128) CK(cudaFuncSetAttribute(k_pf_attention_mma<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pm_smem_bytes<128>()));
@@ -1112,7 +1136,7 @@ int prefill_init(b200_plan *p) {
 int build_f16_twins(b200_plan *p) {
     const b200_config &c = p->cfg;
     if (p->f16_copies) return B200_OK;
-    if (p->wtype != B200_GGML_Q8_0 || !p->use_stream || c.tp_size > 1) return fail(p, B200_ERR_UNSUPPORTED, "f16 twins need a single-GPU Q8_0 plan on the streaming path");
+    if (p->path != Q8_TILES || c.tp_size > 1) return fail(p, B200_ERR_UNSUPPORTED, "f16 twins need a single-GPU Q8_0 plan on the streaming path");
     for (int l = 0; l < c.n_layers; l++) {
         LayerW &L = p->layers[l];
         int rc;
@@ -1135,40 +1159,47 @@ int build_f16_twins(b200_plan *p) {
     return B200_OK;
 }
 
+// One prefill GEMM over n tokens: C[n][N] (MODE: =, += or gate/up SwiGLU) from the A activations and the B (and B2) weight maps, K deep.
+// CTA pairs (c.pair): M in 256-row pair tiles; QKV and gate/up on the persistent kernel, the x += A W^T GEMMs split K so that the
+// grid fills the SMs -- every split reduce-adds its partial product through TMA.  Single CTAs: a GEMM that fits one wave has one
+// CTA per SM anyway and gets the deep ring; otherwise two CTAs share an SM.  A gate/up tile covers half as many output columns.
+template <int MODE>
+int pf_gemm(b200_plan *p, int n, const CUtensorMap &a, const CUtensorMap &b, const CUtensorMap &b2, const CUtensorMap &c_map, void *C, int N, int K) {
+    const int gu = MODE == pg::GEMM_GATEUP ? 2 : 1;
+    cudaStream_t s = p->stream;
+    if (p->prefill.pair) {
+        const int mt2 = (n + 255) / 256 * 2, nt = N * gu / 256;
+        if constexpr (MODE == pg::GEMM_RESID) {
+            const int ctas = mt2 * nt, nk = K / pg::BK;
+            int splits = p->n_sms / ctas;
+            if (splits > 4) splits = 4;
+            while (splits > 1 && nk / splits < 8) splits--;
+            return pg::gemm2_launch<256, pg::GEMM2_STAGES_256>(a, b, c_map, n, mt2, nt, K, s, splits < 1 ? 1 : splits);
+        } else {
+            return pg::gemm2_persist_launch<MODE, 256, pg::GEMM2_PERSIST_STAGES_256>(a, b, b2, c_map, C, N, n, mt2, nt, K, p->n_sms, s);
+        }
+    }
+    const int mt = (n + pg::BM - 1) / pg::BM, nt = N * gu / pg::BN;
+    if (mt * nt <= p->n_sms) return pg::gemm_launch<MODE, pg::GEMM_STAGES_DEEP>(a, b, b2, c_map, C, N, n, mt, nt, K, s);
+    return pg::gemm_launch<MODE, pg::GEMM_STAGES>(a, b, b2, c_map, C, N, n, mt, nt, K, s);
+}
+
 // n tokens already in c.tok (device), positions start_pos .. start_pos + n - 1
 int prefill_forward(b200_plan *p, int n, int start_pos, int *launches) {
     PrefillCtx &c = p->prefill;
     const b200_config &g = p->cfg;
     cudaStream_t s = p->stream;
-    const int nqkv = p->qd + 2 * p->kvd, mt = (n + pg::BM - 1) / pg::BM, kv_mul = g.n_heads / g.n_kv_heads;
+    const int nqkv = p->qd + 2 * p->kvd, kv_mul = g.n_heads / g.n_kv_heads;
     const size_t ctx_kv = (size_t)g.context_length * p->kvd;
     const float inv_sqrt_hs = (float)(1.0 / sqrt((double)g.head_size));
     int nl = 0;
-    constexpr int ST = pg::GEMM_STAGES, DEEP = pg::GEMM_STAGES_DEEP;
-    // a GEMM that fits one wave has one CTA per SM anyway: give it the deep ring; otherwise two CTAs share an SM
-    auto one_wave = [&](int n_tiles) { return mt * n_tiles <= p->n_sms; };
-    // CTA-pair path: M in 256-row pair tiles; QKV and gate/up on the persistent kernel, the x += A W^T GEMMs (N = dim only) split K
-    // so that the grid fills the SMs -- every split reduce-adds its partial product through TMA
-    const int mt2 = (n + 255) / 256 * 2;
-    auto pair_splits = [&](int n_tiles, int K) {
-        const int ctas = mt2 * n_tiles, nk = K / pg::BK;
-        int sp = p->n_sms / ctas;
-        if (sp > 4) sp = 4;
-        while (sp > 1 && nk / sp < 8) sp--;
-        return sp < 1 ? 1 : sp;
-    };
     k_pf_embed<<<n, 256, 0, s>>>(c.tok, p->emb, c.X, g.dim); nl++;
     for (int l = 0; l < g.n_layers; l++) {
         const LayerW &L = p->layers[l];
         const PrefillLayerMaps &m = c.maps[l];
         float *kc = p->key_cache + (size_t)l * ctx_kv, *vc = p->value_cache + (size_t)l * ctx_kv;
         k_pf_rmsnorm_f16<<<n, 256, 0, s>>>(c.X, L.attn_norm, g.rms_norm_eps, g.dim, c.A16); nl++;
-        if (c.pair) {
-            if (pg::gemm2_persist_launch<pg::GEMM_F32, 256, pg::GEMM2_PERSIST_STAGES_256>(c.mA, m.qkv, m.qkv, c.mQKV, c.QKV, nqkv, n, mt2, nqkv / 256, g.dim, p->n_sms, s)) return fail(p, B200_ERR_CUDA, "QKV GEMM launch failed");
-        } else
-        if (one_wave(nqkv / pg::BN) ? pg::gemm_launch<pg::GEMM_F32, DEEP>(c.mA, m.qkv, m.qkv, c.mQKV, c.QKV, nqkv, n, mt, nqkv / pg::BN, g.dim, s)
-                                    : pg::gemm_launch<pg::GEMM_F32, ST>(c.mA, m.qkv, m.qkv, c.mQKV, c.QKV, nqkv, n, mt, nqkv / pg::BN, g.dim, s))
-            return fail(p, B200_ERR_CUDA, "QKV GEMM launch failed");
+        if (pf_gemm<pg::GEMM_F32>(p, n, c.mA, m.qkv, m.qkv, c.mQKV, c.QKV, nqkv, g.dim)) return fail(p, B200_ERR_CUDA, "QKV GEMM launch failed");
         nl++;
         const int qt = PM_ROWS / kv_mul;
         const dim3 ag((n + qt - 1) / qt, g.n_kv_heads);
@@ -1185,29 +1216,12 @@ int prefill_forward(b200_plan *p, int n, int start_pos, int *launches) {
             k_pf_attention_mma<64><<<ag, PM_THREADS, pm_smem_bytes<64>(), s>>>(c.QKV, nqkv, c.KH, c.VH, p->kvd, kv_mul, n, start_pos, inv_sqrt_hs, c.ATT16, p->qd);
         }
         nl += 2;
-        if (c.pair) {
-            if (pg::gemm2_launch<256, pg::GEMM2_STAGES_256>(c.mATT, m.wo, c.mX, n, mt2, g.dim / 256, p->qd, s, pair_splits(g.dim / 256, p->qd)))
-                return fail(p, B200_ERR_CUDA, "Wo GEMM launch failed");
-        } else
-        if (one_wave(g.dim / pg::BN) ? pg::gemm_launch<pg::GEMM_RESID, DEEP>(c.mATT, m.wo, m.wo, c.mX, c.X, g.dim, n, mt, g.dim / pg::BN, p->qd, s)
-                                     : pg::gemm_launch<pg::GEMM_RESID, ST>(c.mATT, m.wo, m.wo, c.mX, c.X, g.dim, n, mt, g.dim / pg::BN, p->qd, s))
-            return fail(p, B200_ERR_CUDA, "Wo GEMM launch failed");
+        if (pf_gemm<pg::GEMM_RESID>(p, n, c.mATT, m.wo, m.wo, c.mX, c.X, g.dim, p->qd)) return fail(p, B200_ERR_CUDA, "Wo GEMM launch failed");
         nl++;
         k_pf_rmsnorm_f16<<<n, 256, 0, s>>>(c.X, L.ffn_norm, g.rms_norm_eps, g.dim, c.A16); nl++;
-        if (c.pair) {
-            if (pg::gemm2_persist_launch<pg::GEMM_GATEUP, 256, pg::GEMM2_PERSIST_STAGES_256>(c.mA, m.w1p, m.w3p, c.mX, c.H16, g.hidden_dim, n, mt2, g.hidden_dim / 128, g.dim, p->n_sms, s)) return fail(p, B200_ERR_CUDA, "gate/up GEMM launch failed");
-        } else
-        if (one_wave(g.hidden_dim / (pg::BN / 2)) ? pg::gemm_launch<pg::GEMM_GATEUP, DEEP>(c.mA, m.w1, m.w3, c.mX, c.H16, g.hidden_dim, n, mt, g.hidden_dim / (pg::BN / 2), g.dim, s)
-                                                  : pg::gemm_launch<pg::GEMM_GATEUP, ST>(c.mA, m.w1, m.w3, c.mX, c.H16, g.hidden_dim, n, mt, g.hidden_dim / (pg::BN / 2), g.dim, s))
-            return fail(p, B200_ERR_CUDA, "gate/up GEMM launch failed");
+        if (pf_gemm<pg::GEMM_GATEUP>(p, n, c.mA, m.w1, m.w3, c.mX, c.H16, g.hidden_dim, g.dim)) return fail(p, B200_ERR_CUDA, "gate/up GEMM launch failed");
         nl++;
-        if (c.pair) {
-            if (pg::gemm2_launch<256, pg::GEMM2_STAGES_256>(c.mH, m.w2, c.mX, n, mt2, g.dim / 256, g.hidden_dim, s, pair_splits(g.dim / 256, g.hidden_dim)))
-                return fail(p, B200_ERR_CUDA, "W2 GEMM launch failed");
-        } else
-        if (one_wave(g.dim / pg::BN) ? pg::gemm_launch<pg::GEMM_RESID, DEEP>(c.mH, m.w2, m.w2, c.mX, c.X, g.dim, n, mt, g.dim / pg::BN, g.hidden_dim, s)
-                                     : pg::gemm_launch<pg::GEMM_RESID, ST>(c.mH, m.w2, m.w2, c.mX, c.X, g.dim, n, mt, g.dim / pg::BN, g.hidden_dim, s))
-            return fail(p, B200_ERR_CUDA, "W2 GEMM launch failed");
+        if (pf_gemm<pg::GEMM_RESID>(p, n, c.mH, m.w2, m.w2, c.mX, c.X, g.dim, g.hidden_dim)) return fail(p, B200_ERR_CUDA, "W2 GEMM launch failed");
         nl++;
     }
     CK(cudaGetLastError());
@@ -1422,7 +1436,7 @@ int b200_trace_persistent(b200_plan *p, int32_t token, int32_t position, uint64_
 
 int b200_set_prefill_mode(b200_plan *p, int32_t mode) {
     if (!p || (mode != B200_PREFILL_EXACT && mode != B200_PREFILL_TENSOR_CORE)) return B200_ERR_BAD_ARG;
-    if (mode == B200_PREFILL_TENSOR_CORE && !p->prefill.ready && p->prefill_batch > 1 && p->wtype == B200_GGML_Q8_0 && p->use_stream && p->cfg.tp_size == 1) {
+    if (mode == B200_PREFILL_TENSOR_CORE && !p->prefill.ready && p->prefill_batch > 1 && p->path == Q8_TILES && p->cfg.tp_size == 1) {
         CK(cudaSetDevice(p->device)); // opt-in on a Q8_0 plan: build the f16 twins, then the GEMM context
         int rc = build_f16_twins(p);
         if (rc) return rc;
@@ -1482,99 +1496,29 @@ int b200_read_buffer(b200_plan *p, const char *name, int32_t layer, void *dst, s
 int b200_time_kernel(b200_plan *p, int32_t which, int32_t reps, float *avg_ms, int64_t *algorithmic_bytes) {
     if (!p || !avg_ms || reps <= 0) return B200_ERR_BAD_ARG;
     if (p->cfg.tp_size > 1) return fail(p, B200_ERR_UNSUPPORTED, "b200_time_kernel is single-GPU only");
+    if (which < MV_GATEUP || which > MV_CLS) return fail(p, B200_ERR_BAD_ARG, "unknown kernel id %d", which);
     const b200_config &c = p->cfg;
-    const bool q8 = p->wtype == B200_GGML_Q8_0;
+    const MvRole role = (MvRole)which;
     CK(cudaSetDevice(p->device));
     std::vector<float> save(c.dim);
     CK(cudaStreamSynchronize(p->stream));
     CK(cudaMemcpy(save.data(), p->x, (size_t)c.dim * 4, cudaMemcpyDeviceToHost));
-    if (p->use_stream) {
-        auto tb = [&](const TileMat &m) -> int64_t { return (int64_t)m.rows * m.cols / 32 * 34; };
-        int64_t bytes = 0;
-        int launches = 0, rc;
-        auto one = [&](int l) -> int {
-            LayerW &L = p->layers[l];
-            bool keep = p->use_pdl;
-            p->use_pdl = false;
-            int r;
-            switch (which) {
-            case 0: bytes = tb(L.tgu); r = launch_stream<SMV_GATEUP>(p, L.tgu, p->xq, p->xs, p->hb, p->hq, p->hs); break;
-            case 1: bytes = tb(L.tw2); r = launch_stream<SMV_RESID>(p, L.tw2, p->hq, p->hs, p->x, nullptr, nullptr); break;
-            case 2: bytes = tb(L.tqkv); r = launch_stream<SMV_STORE>(p, L.tqkv, p->xq, p->xs, p->qkv, nullptr, nullptr); break;
-            case 3: bytes = tb(L.two); r = launch_stream<SMV_RESID>(p, L.two, p->xq, p->xs, p->x, nullptr, nullptr); break;
-            default: bytes = tb(p->tout); r = launch_stream<SMV_STORE>(p, p->tout, p->xq, p->xs, p->logits, nullptr, nullptr); break;
-            }
-            p->use_pdl = keep;
-            return r;
-        };
-        if (which < 0 || which > 4) return fail(p, B200_ERR_BAD_ARG, "unknown kernel id %d", which);
-        for (int l = 0; l < c.n_layers; l++) if ((rc = one(l))) return rc;
-        CK(cudaEventRecord(p->ev0, p->stream));
-        for (int r = 0; r < reps; r++)
-            for (int l = 0; l < c.n_layers; l++) { if ((rc = one(l))) return rc; launches++; }
-        CK(cudaEventRecord(p->ev1, p->stream));
-        CK(cudaStreamSynchronize(p->stream));
-        float ms = 0;
-        CK(cudaEventElapsedTime(&ms, p->ev0, p->ev1));
-        *avg_ms = ms / launches;
-        if (algorithmic_bytes) *algorithmic_bytes = bytes;
-        CK(cudaMemcpy(p->x, save.data(), (size_t)c.dim * 4, cudaMemcpyHostToDevice));
-        return B200_OK;
-    }
-    auto mat_bytes = [&](const DevMat &m) -> int64_t {
-        int64_t e = (int64_t)m.rows * m.cols;
-        return q8 ? e / 32 * 34 : e * 2;
-    };
-    int64_t bytes = 0;
-    int launches = 0;
-    const bool sf = p->use_f16_stream;
-    auto one = [&](int l) -> int {
-        LayerW &L = p->layers[l];
-        if (sf) { // FP16 streaming kernels, stand-alone (no PDL overlap)
-            const bool keep = p->use_pdl;
-            p->use_pdl = false;
-            int r;
-            switch (which) {
-            case 0: bytes = mat_bytes(L.w1) + mat_bytes(L.w3); r = launch_stream_f16<SF_GATEUP>(p, L.w1, &L.w3, p->xb, p->hb); break;
-            case 1: bytes = mat_bytes(L.w2); r = launch_stream_f16<SF_RESID>(p, L.w2, nullptr, p->hb, p->x); break;
-            case 2: bytes = mat_bytes(L.qkv); r = launch_stream_f16<SF_STORE>(p, L.qkv, nullptr, p->xb, p->qkv); break;
-            case 3: bytes = mat_bytes(L.wo); r = launch_stream_f16<SF_RESID>(p, L.wo, nullptr, p->xb, p->x); break;
-            default: bytes = mat_bytes(p->out); r = launch_stream_f16<SF_STORE>(p, p->out, nullptr, p->xb, p->logits); break;
-            }
-            p->use_pdl = keep;
-            return r;
-        }
-        switch (which) {
-        case 0:
-            if (q8) {
-                k_gateup_q8<<<c.hidden_dim / 32, 256, q8_smem_bytes(c.dim, 4, 8), p->stream>>>(
-                    (const int8_t *)L.w1.qs, L.w1.sc, (const int8_t *)L.w3.qs, L.w3.sc, p->xq, p->xs, c.hidden_dim, c.dim, p->hq, p->hs, p->hb);
-                CK(cudaGetLastError());
-            } else {
-                int rc;
-                if ((rc = launch_matvec_f16<MODE_STORE>(p, L.w1, p->xb, p->hb))) return rc;
-                if ((rc = launch_matvec_f16<MODE_STORE>(p, L.w3, p->xb, p->hb2))) return rc;
-            }
-            bytes = mat_bytes(L.w1) + mat_bytes(L.w3);
-            return B200_OK;
-        case 1: bytes = mat_bytes(L.w2); return q8 ? launch_matvec_q8<MODE_RESID>(p, L.w2, p->hq, p->hs, p->x) : launch_matvec_f16<MODE_RESID>(p, L.w2, p->hb, p->x);
-        case 2: bytes = mat_bytes(L.qkv); return q8 ? launch_matvec_q8<MODE_STORE>(p, L.qkv, p->xq, p->xs, p->qkv) : launch_matvec_f16<MODE_STORE>(p, L.qkv, p->xb, p->qkv);
-        case 3: bytes = mat_bytes(L.wo); return q8 ? launch_matvec_q8<MODE_RESID>(p, L.wo, p->xq, p->xs, p->x) : launch_matvec_f16<MODE_RESID>(p, L.wo, p->xb, p->x);
-        default: bytes = mat_bytes(p->out); return q8 ? launch_matvec_q8<MODE_STORE>(p, p->out, p->xq, p->xs, p->logits) : launch_matvec_f16<MODE_STORE>(p, p->out, p->xb, p->logits);
-        }
-    };
-    if (which < 0 || which > 4) return fail(p, B200_ERR_BAD_ARG, "unknown kernel id %d", which);
+    // stand-alone launches (no PDL overlap), one per layer
     int rc;
-    for (int l = 0; l < c.n_layers; l++) if ((rc = one(l))) return rc; // warm-up pass (also defeats L2 for pass 1)
+    for (int l = 0; l < c.n_layers; l++) if ((rc = launch_mv(p, role, l, false, TraceBuf{nullptr, 0, 0})) < 0) return rc; // warm-up pass (also defeats L2 for pass 1)
     CK(cudaEventRecord(p->ev0, p->stream));
     for (int r = 0; r < reps; r++)
-        for (int l = 0; l < c.n_layers; l++) { if ((rc = one(l))) return rc; launches++; }
+        for (int l = 0; l < c.n_layers; l++) if ((rc = launch_mv(p, role, l, false, TraceBuf{nullptr, 0, 0})) < 0) return rc;
     CK(cudaEventRecord(p->ev1, p->stream));
     CK(cudaStreamSynchronize(p->stream));
     float ms = 0;
     CK(cudaEventElapsedTime(&ms, p->ev0, p->ev1));
-    *avg_ms = ms / launches;
-    if (algorithmic_bytes) *algorithmic_bytes = bytes;
+    *avg_ms = ms / (reps * c.n_layers);
+    if (algorithmic_bytes) { // the weight bytes one launch streams
+        const int64_t rows[5] = {2LL * c.hidden_dim, c.dim, p->qd + 2LL * p->kvd, c.dim, c.vocab_size}, cols[5] = {c.dim, c.hidden_dim, c.dim, p->qd, c.dim};
+        const int64_t e = rows[role] * cols[role];
+        *algorithmic_bytes = p->wtype == B200_GGML_Q8_0 ? e / 32 * 34 : e * 2;
+    }
     CK(cudaMemcpy(p->x, save.data(), (size_t)c.dim * 4, cudaMemcpyHostToDevice));
     return B200_OK;
 }
@@ -1680,13 +1624,11 @@ int b200_requant_kquant(int32_t ggml_type, const void *src, int64_t n_elems, voi
     return rc;
 }
 
-int b200_gemm_f16(const uint16_t *a, const uint16_t *b, float *c, int32_t m, int32_t n, int32_t k, int32_t iters, float *ms) {
-    const int stages = getenv("B200_GEMM_STAGES") ? atoi(getenv("B200_GEMM_STAGES")) : 0;
-    const int two_cta = getenv("B200_GEMM_2CTA") ? atoi(getenv("B200_GEMM_2CTA")) : 0; // 0, 256 (with B200_GEMM_RESID) or 1256 (without)
-    const int resid = getenv("B200_GEMM_RESID") ? atoi(getenv("B200_GEMM_RESID")) : 0; // C starts at 0 and accumulates over the timed launches
+int b200_gemm_f16(const uint16_t *a, const uint16_t *b, float *c, int32_t m, int32_t n, int32_t k, int32_t iters, float *ms, int32_t stages,
+                  int32_t resid, int32_t two_cta) {
     if (!a || !b || !c || m <= 0 || n <= 0 || k <= 0 || m % 128 || n % 128 || k % 64) return B200_ERR_BAD_ARG;
-    // only the kernels the prefill launches (pg::gemm_f16)
-    if (two_cta ? two_cta != (resid ? 256 : 1256) : (stages != 0 && stages != 3 && stages != 6)) return B200_ERR_BAD_ARG;
+    // only the kernels the prefill launches (pg::gemm_f16); with resid, C starts at 0 and accumulates over the timed launches
+    if (resid < 0 || (two_cta ? two_cta != (resid ? 256 : 1256) : (stages != 0 && stages != 3 && stages != 6))) return B200_ERR_BAD_ARG;
     __half *da = nullptr, *db = nullptr;
     float *dc = nullptr;
     cudaEvent_t e0 = nullptr, e1 = nullptr;

@@ -25,15 +25,14 @@
 #include <vector>
 
 struct PrefillLayerMaps {
-    CUtensorMap qkv, wo, w1, w3, w2; // weight boxes of 128 rows (64 for w1 / w3: the single-CTA gate/up tile is 64 + 64)
-    CUtensorMap w1p, w3p;            // 128-row boxes for the CTA-pair gate/up tile (128 + 128)
+    CUtensorMap qkv, wo, w1, w3, w2; // weight boxes of 128 rows; w1 / w3: 128 on CTA pairs, 64 on single CTAs (gate/up tile 64 + 64)
 };
 
 struct PrefillCtx {
     int batch = 0, bpad = 0;
     bool ready = false; // tensor-core path usable for this plan
     int mode = 0;       // 0 = exact token-by-token graph, 1 = tensor-core GEMMs
-    bool pair = true;      // CTA-pair (cta_group::2) GEMMs; B200_GEMM_2CTA=0 selects the single-CTA kernels
+    bool pair = true;      // CTA-pair (cta_group::2) GEMMs; single-CTA ones for shapes the 256-wide pair tiles do not divide
     float *X = nullptr, *QKV = nullptr;
     __half *A16 = nullptr, *ATT16 = nullptr, *H16 = nullptr;
     int *tok = nullptr;

@@ -72,7 +72,7 @@ def lib() -> C.CDLL:
     L.b200_trace_persistent.argtypes = [vp, i32, i32, vp, C.c_int64, C.POINTER(i32), C.POINTER(i32), C.POINTER(i32)]
     L.b200_test_seqsum2.argtypes = [vp, i32, i32, C.POINTER(C.c_float), C.POINTER(i32)]
     L.b200_prefill_info.argtypes = [vp, C.POINTER(i32), C.POINTER(i32), C.POINTER(C.c_float)]
-    L.b200_gemm_f16.argtypes = [vp, vp, vp, i32, i32, i32, i32, C.POINTER(C.c_float)]
+    L.b200_gemm_f16.argtypes = [vp, vp, vp, i32, i32, i32, i32, C.POINTER(C.c_float), i32, i32, i32]
     L.b200_time_kernel.argtypes = [vp, i32, i32, C.POINTER(C.c_float), C.POINTER(C.c_int64)]
     L.b200_read_buffer.argtypes = [vp, C.c_char_p, i32, vp, C.c_size_t]
     L.b200_upload_info.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_int64)]
@@ -116,8 +116,9 @@ def requant_kquant(ggml_type: int, raw, n_elems: int) -> np.ndarray:
     return out
 
 
-def gemm_f16(a, b, iters: int = 0):
-    """C = A @ B.T on the tcgen05 prefill GEMM (A [m,k], B [n,k] float16) -> (C float32, ms per launch or None)."""
+def gemm_f16(a, b, iters: int = 0, stages: int = 0, resid: int = 0, two_cta: int = 0):
+    """C = A @ B.T on the tcgen05 prefill GEMM (A [m,k], B [n,k] float16) -> (C float32, ms per launch or None).
+    stages / resid / two_cta pick the prefill kernel as include/b200llama.h documents for b200_gemm_f16."""
     a = np.ascontiguousarray(a, dtype=np.float16)
     b = np.ascontiguousarray(b, dtype=np.float16)
     m, k = a.shape
@@ -126,7 +127,7 @@ def gemm_f16(a, b, iters: int = 0):
         raise ValueError("inner dimensions differ")
     c = np.empty((m, n), dtype=np.float32)
     ms = C.c_float(0)
-    rc = lib().b200_gemm_f16(a.ctypes.data, b.ctypes.data, c.ctypes.data, m, n, k, iters, C.byref(ms))
+    rc = lib().b200_gemm_f16(a.ctypes.data, b.ctypes.data, c.ctypes.data, m, n, k, iters, C.byref(ms), stages, resid, two_cta)
     if rc != B200_OK:
         _raise(rc, "b200_gemm_f16 failed")
     return c, (ms.value if iters > 0 else None)

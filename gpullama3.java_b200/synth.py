@@ -51,6 +51,10 @@ SHAPES = {
     "tiny-llama": Shape("llama", 256, 512, 2, 4, 2, 64, 512, False, 500000.0, 1e-5),
     "tiny-llama-tied": Shape("llama", 256, 512, 2, 4, 2, 64, 512, True, 500000.0, 1e-5),
     "tiny-qwen3": Shape("qwen3", 256, 768, 2, 4, 2, 128, 640, True, 1000000.0, 1e-6),
+    # shapes the fast decode layouts do not fit: a classifier of 510 rows (not a multiple of 4) keeps a Q8_0 plan off the tile
+    # stream; dim 384 (not a multiple of 256) keeps an FP16 plan off the rings and its prefill off the CTA-pair GEMMs
+    "tiny-llama-odd-vocab": Shape("llama", 256, 512, 2, 4, 2, 64, 510, False, 500000.0, 1e-5),
+    "tiny-llama-384": Shape("llama", 384, 1024, 2, 6, 3, 64, 512, False, 500000.0, 1e-5),
     # Phi-3 (forwardJavaPhi3: fused attn_qkv / gate-up tensors, NeoX-pair RoPE): mini-like (multi-head, head size 96) and medium-like (GQA, 128)
     "tiny-phi3": Shape("phi3", 384, 768, 2, 4, 4, 96, 512, False, 10000.0, 1e-5, 4096),
     "tiny-phi3-gqa": Shape("phi3", 512, 1024, 2, 4, 2, 128, 512, False, 10000.0, 1e-5, 4096),

@@ -181,7 +181,9 @@ int b200_read_buffer(b200_plan *plan, const char *name, int32_t layer, void *dst
  * stand-alone, `reps` times per layer, cycling over all layers so every launch streams weights
  * that are not L2-resident, and returns the average duration of one launch (CUDA events on the
  * plan's stream).  which: 0 = fused gate/up+SwiGLU, 1 = down projection (+residual),
- * 2 = fused QKV, 3 = attention output projection (+residual), 4 = lm_head.
+ * 2 = fused QKV, 3 = attention output projection (+residual), 4 = lm_head.  Each id launches what the
+ * decode step launches for that matrix, without programmatic dependent launch (on the FP16 row
+ * kernels gate/up is three launches: w1, w3 and the SwiGLU).
  * The residual stream is restored afterwards; the KV cache is not touched. */
 int b200_time_kernel(b200_plan *plan, int32_t which, int32_t reps, float *avg_ms, int64_t *algorithmic_bytes);
 
@@ -227,12 +229,12 @@ int b200_requant_kquant(int32_t ggml_type, const void *src, int64_t n_elems, voi
  * gemmMMA / gemmMMAQKV / gemmMMAGateUp, TransformerBatchPrefillKernels.java:792-1132) exposed for
  * tests and measurement: C[m][n] (f32) = A[m][k] (f16 bits) x B[n][k]^T (f16 bits) on tcgen05 tensor
  * cores, FP32 accumulation in TMEM.  Host pointers; m % 128 == n % 128 == k % 64 == 0.
- * The kernel is one the prefill launches, chosen by B200_GEMM_2CTA / B200_GEMM_RESID / B200_GEMM_STAGES: 0 = single-CTA
- * (C = A B^T, or C += A B^T with B200_GEMM_RESID=1; 3 or 6 stages), 256 = CTA-pair C += A B^T split B200_GEMM_RESID ways over k
- * (needs B200_GEMM_RESID >= 1), 1256 = persistent CTA-pair C = A B^T (needs B200_GEMM_RESID unset or 0); CTA-pair kernels need
- * m % 256 == n % 256 == 0.  Any other combination returns B200_ERR_BAD_ARG.
+ * The kernel is one the prefill launches, chosen by two_cta: 0 = single-CTA (C = A B^T, or C += A B^T with resid = 1;
+ * stages 3 or 6, 0 = 3), 256 = CTA-pair C += A B^T split `resid` ways over k (needs resid >= 1), 1256 = persistent CTA-pair
+ * C = A B^T (needs resid == 0); CTA-pair kernels need m % 256 == n % 256 == 0.  Any other combination returns B200_ERR_BAD_ARG.
  * iters > 0 additionally times `iters` back-to-back launches (device events) into *ms. */
-int b200_gemm_f16(const uint16_t *a, const uint16_t *b, float *c, int32_t m, int32_t n, int32_t k, int32_t iters, float *ms /* nullable */);
+int b200_gemm_f16(const uint16_t *a, const uint16_t *b, float *c, int32_t m, int32_t n, int32_t k, int32_t iters, float *ms /* nullable */,
+                  int32_t stages, int32_t resid, int32_t two_cta);
 
 /* Weight upload of b200_plan_create (the counterpart of the reference's load-time metrics, ModelLoader.java:102-106 and the
  * copy-in timing of TornadoVMMasterPlanSingleToken.java:51-54): wall seconds from the first tensor to the last repack kernel,

@@ -42,11 +42,14 @@ def _requantised_twin(pkg, orc, m):
     return pkg.loader.Model(None, m.configuration, m.model_type, tensors)
 
 
-def _decode_matches(pkg, orc, m, n_tok, mode=None):
+def _decode_matches(pkg, orc, m, n_tok, mode=None, rows=False):
     c = m.configuration
     plan = pkg.B200MasterPlan.initialize_plan(m)
     om = orc.OracleModel(_requantised_twin(pkg, orc, m))
     try:
+        if rows:  # the Q8_0 row kernels: the plan has no tile-major stream, so the persistent kernel is unavailable
+            with pytest.raises(pkg.native.UnsupportedOperation, match="streaming layout"):
+                plan.set_decode_mode("persistent")
         if mode:
             plan.set_decode_mode(mode)
         toks = orc.bench_tokens(c.vocab_size, n_tok)
@@ -72,15 +75,14 @@ def test_kquant_model_decodes_like_its_q8_0_twin(pkg, orc, shape, mix):
     _decode_matches(pkg, orc, m, 10)
 
 
-def test_kquant_model_other_paths(pkg, orc, monkeypatch):
-    """The round-1 non-streaming kernels (B200_STREAM=0: every matrix goes through the chunked split-plane upload) and the
-    persistent decode kernel see the same re-quantised weights."""
-    sh = pkg.synth.SHAPES["tiny-llama"]
-    tensors = pkg.synth.build_tensors_kquant(sh, seed=12)
-    m = pkg.loader.model_from_tensors(sh, pkg.gguf.GGMLType.Q8_0, tensors, 24)
-    _decode_matches(pkg, orc, m, 6, mode="persistent")
-    monkeypatch.setenv("B200_STREAM", "0")
-    _decode_matches(pkg, orc, m, 6)
+def test_kquant_model_other_paths(pkg, orc):
+    """The persistent decode kernel and the Q8_0 row kernels (a 510-row classifier does not fit the tile stream, so every matrix
+    goes through the chunked split-plane upload) see the same re-quantised weights."""
+    for shape, mode, rows in (("tiny-llama", "persistent", False), ("tiny-llama-odd-vocab", None, True)):
+        sh = pkg.synth.SHAPES[shape]
+        tensors = pkg.synth.build_tensors_kquant(sh, seed=12)
+        m = pkg.loader.model_from_tensors(sh, pkg.gguf.GGMLType.Q8_0, tensors, 24)
+        _decode_matches(pkg, orc, m, 6, mode=mode, rows=rows)
 
 
 def test_kquant_real_geometry(pkg, orc):

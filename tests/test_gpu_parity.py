@@ -34,9 +34,11 @@ def set_mode(pkg, plan, mode):
     assert plan.decode_info()[0] == {"graph": 0, "persistent": 1}[mode]
 
 
-def run_stream(pkg, orc, model, lanes, n, check_kv=True, prefill_first=0, mode="graph"):
+def run_stream(pkg, orc, model, lanes, n, check_kv=True, prefill_first=0, mode="graph", launches=None):
     plan = pkg.B200MasterPlan.initialize_plan(model, fp16_lanes=lanes)
     set_mode(pkg, plan, mode)
+    if launches is not None:  # kernels per decode step: tells the decode paths apart
+        assert plan.launches_per_decode == launches, plan.launches_per_decode
     om = orc.OracleModel(model, lanes=lanes)
     c = model.configuration
     stream = orc.bench_tokens(c.vocab_size, n)
@@ -62,9 +64,20 @@ def run_stream(pkg, orc, model, lanes, n, check_kv=True, prefill_first=0, mode="
 
 
 @pytest.mark.parametrize("mode", MODES)
-@pytest.mark.parametrize("shape", ["tiny-llama", "tiny-llama-tied", "tiny-qwen3"])
+@pytest.mark.parametrize("shape", ["tiny-llama", "tiny-llama-tied", "tiny-qwen3", "tiny-llama-odd-vocab"])
 def test_decode_q8_bit_exact(pkg, orc, make_model, shape, mode):
+    """tiny-llama-odd-vocab: its 510-row classifier does not fit the tile stream, so the plan runs the Q8_0 row kernels, and the
+    persistent kernel, which reads the tile stream, is refused."""
     m = make_model(shape, pkg.gguf.GGMLType.Q8_0, 24)
+    if shape == "tiny-llama-odd-vocab":
+        plan = pkg.B200MasterPlan.initialize_plan(m)
+        try:
+            with pytest.raises(pkg.native.UnsupportedOperation, match="streaming layout"):
+                plan.set_decode_mode("persistent")
+        finally:
+            plan.free()
+        if mode == "persistent":
+            return
     run_stream(pkg, orc, m, 16, 20, mode=mode)
 
 
@@ -106,11 +119,11 @@ def test_decode_phi3_mini_geometry(pkg, orc, quant):
     run_stream(pkg, orc, m, 16, 4, check_kv=True)
 
 
-def test_decode_f16_round1_kernels_still_exact(pkg, orc, make_model, monkeypatch):
-    """B200_F16_STREAM=0 keeps the round-1 launches (k_matvec_f16 + separate SwiGLU), the fallback for shapes the rings do not fit."""
-    monkeypatch.setenv("B200_F16_STREAM", "0")
-    m = make_model("tiny-llama", pkg.gguf.GGMLType.F16, 24)
-    run_stream(pkg, orc, m, 16, 8)
+def test_decode_f16_round1_kernels_still_exact(pkg, orc, make_model):
+    """The round-1 launches (k_matvec_f16 + separate SwiGLU), the fallback for shapes the rings do not fit: dim 384 is not a
+    multiple of the rings' 256-column segments.  They issue 9 launches per layer where the rings issue 7."""
+    m = make_model("tiny-llama-384", pkg.gguf.GGMLType.F16, 24)
+    run_stream(pkg, orc, m, 16, 8, launches=9 * m.configuration.n_layers + 3)
 
 
 @pytest.mark.parametrize("mode", MODES)
